@@ -19,6 +19,9 @@ load f = 2 pi^2 sin(pi x) sin(pi y)) into CSR values + load vector.  Prints ONE 
 the GPU box; see DESIGN.md).  Multi-GPU (`torchrun`, one rank per GPU): weak scaling, each rank
 assembles its own 4.19 M-element strip of a mesh that is N times taller; interface rows travel
 over NVLink peer memory while the interior assembles (DESIGN.md section 6).
+
+`--dump-outputs DIR` writes the CSR values and the load vector of the last timed step to DIR (see
+`dump_outputs`), so that two builds can be compared output for output on the same seeded mesh.
 """
 
 from __future__ import annotations
@@ -55,7 +58,12 @@ def parse_args():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--permuted", action="store_true",
                    help="locality stress (SURVEY.md 8(d)): random renumbering of vertices and elements, default_rng(7); N=1 only")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="write the CSR values and load vector of the last timed step as DIR/csr_values.npy and DIR/load.npy; one GPU only")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def measured_peak():
@@ -124,6 +132,28 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": ordered[len(ordered) // 2], "sm_max_mhz": self.max_mhz, "reasons": sorted(self.reasons), "samples": len(ordered)}
 
 
+DUMP_MAX_BYTES = 64_000_000  # both files together, .npy headers included
+# per array: half the budget, less room for its .npy header (128 bytes for a 1-D float64 array)
+DUMP_MAX_ELEMENTS = (DUMP_MAX_BYTES // 2 - 4096) // 8
+
+
+def dump_outputs(directory, values, load):
+    """Write the CSR values and the load vector as DIR/csr_values.npy and DIR/load.npy (1-D float64).
+
+    An array longer than DUMP_MAX_ELEMENTS is replaced by its entries at the sorted indices of
+    `numpy.random.default_rng(0).choice(length, DUMP_MAX_ELEMENTS, replace=False)`: the same entries on every run
+    of the same mesh, so the dumps of two builds (or of `--impl ours` and `--impl reference`, whose CSR patterns
+    are the same) compare entry for entry."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, array in (("csr_values", values), ("load", load)):
+        flat = array.detach().reshape(-1).cpu().numpy().astype(np.float64, copy=False)
+        if flat.size > DUMP_MAX_ELEMENTS:
+            flat = flat[np.sort(np.random.default_rng(0).choice(flat.size, DUMP_MAX_ELEMENTS, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), flat)
+
+
 def cpu_reference_run(nx, ny, repeats=1):
     """Time the CPU port of the reference pipeline; returns (elements/s, description, timings)."""
     import torch
@@ -165,9 +195,14 @@ def run_reference(args):
     for _ in range(args.warmup):
         reference_assembly_cpu(coords, conn, QUAD_ORDER)
     t0 = time.perf_counter()
-    for _ in range(args.steps):
-        reference_assembly_cpu(coords, conn, QUAD_ORDER)
+    for i in range(args.steps):
+        last = reference_assembly_cpu(coords, conn, QUAD_ORDER)
+        if i + 1 < args.steps:
+            last = None  # only the last step's outputs are kept
     elapsed = time.perf_counter() - t0
+    if args.dump_outputs:
+        matrix, load = last
+        dump_outputs(args.dump_outputs, matrix.values(), load)
     value = n_el * args.steps / elapsed
     cores = torch.get_num_threads()
     sample = f"all {n_el} elements per step (nx={nx}, ny={ny}); {args.warmup} warm-up + {args.steps} timed steps"
@@ -222,6 +257,8 @@ def run_ours(args):
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the outputs of one GPU: run it with --gpus 1")
     torch.cuda.set_device(local_rank)
     device = torch.device("cuda", local_rank)
     if world > 1:
@@ -295,7 +332,7 @@ def run_ours(args):
         plan = None
 
         def local_step():
-            basis._assemble_fused(bilinear, src, "two_pass")
+            return basis._assemble_fused(bilinear, src, "two_pass")
 
         kernels_per_step = 3
 
@@ -338,14 +375,25 @@ def run_ours(args):
     for i in range(args.steps):
         flush.fill_(float(i))  # evict L2 (126 MB) between timed steps; outside the event pair
         starts[i].record()
-        step()
+        last = step()
         ends[i].record()
+        if i + 1 < args.steps:
+            last = None  # only the last step's outputs are kept; earlier ones go back to the allocator as before
     barrier()
     sampler.active = False
     gpu_launches = sum(_lib.LAUNCHES.values()) - launches_before
     times_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]
     total_ms = sum(times_ms)
     clocks = sampler.stop()
+    # the tiled step writes into `values` / `load`, the two-pass step returns fresh arrays; a device copy is
+    # written to disk after every timed phase, so the host work of the dump cannot idle the GPU between them
+    dumped = None
+    if args.dump_outputs:
+        if args.path == "two_pass":
+            dumped = [t.clone() for t in last]
+        else:
+            dumped = [values.clone(), load.clone()]
+    del last
 
     # kernel-only time of the dominant kernel (roofline numerator), same stream, same flush
     k_ms = []
@@ -415,6 +463,8 @@ def run_ours(args):
     if world > 1:
         dist.all_reduce(stats, op=dist.ReduceOp.MAX)
     total_ms, kernel_ms, e2e_step_s = stats.tolist()
+    if dumped is not None:
+        dump_outputs(args.dump_outputs, *dumped)
     strong = world > 1 and args.scaling == "strong"
     total_elements = 2 * args.nx * args.ny if strong else n_el * world
 
