@@ -152,6 +152,30 @@ int tfem_set_device(int device);
 /* Number of SMs of the current device (grid sizing of persistent kernels; 148 on B200). */
 int tfem_sm_count(void);
 
+/* One smoothed level of an AMG hierarchy (pytorch_fem_solver_b200/sparse.py `amg`; DESIGN.md 8(f).1), all pointers
+ * DEVICE memory in the precision of the call (T = double for _f64, float for _f32).  Level l holds its operator
+ * A [n x n], the prolongator P [n x n_coarse] and restriction R = P^T [n_coarse x n] as CSR (int32 crow / col),
+ * wdinv [n] = omega / a_ii, and work vectors x [n] (the level's smoothed iterate), rc [n_coarse] (restricted
+ * residual = right-hand side of level l + 1) and ec [n_coarse] (its correction = result of level l + 1).
+ * n_coarse equals the n of the next level, or of the dense coarsest operator after the last level. */
+typedef struct tfem_amg_level {
+  int64_t n;
+  int64_t n_coarse;
+  const int32_t* a_crow;
+  const int32_t* a_col;
+  const void* a_val;
+  const int32_t* p_crow;
+  const int32_t* p_col;
+  const void* p_val;
+  const int32_t* r_crow;
+  const int32_t* r_col;
+  const void* r_val;
+  const void* wdinv;
+  void* x;
+  void* rc;
+  void* ec;
+} tfem_amg_level;
+
 #define TFEM_DECLARE(T, SUF)                                                                        \
   /* a1-a9: AbstractBasis._compute_integral_values (basis/abstract_basis.py:42-63) with          \
    * Basis._compute_jacobian_map/_integration_points/_integral_weights (basis/basis.py:87-96),   \
@@ -318,6 +342,46 @@ int tfem_sm_count(void);
   int tfem_cg_iteration_##SUF(int64_t n, const int32_t* crow, const int32_t* col, const T* val,    \
                               const uint8_t* keep, const T* inv_diag, T* x, T* r, T* z, T* p,      \
                               T* ap, T* partial, int32_t n_partial, T* scal, void* stream);      \
+  /* The same iteration preconditioned by smoothed-aggregation AMG instead of Jacobi: SpMV + p.Ap   \
+   * (the kernel of tfem_cg_iteration), x += alpha p and r -= alpha ap, z = M_AMG r (one V-cycle,   \
+   * as tfem_amg_vcycle), partials of r.z, the new direction.  Same state and scal contract as      \
+   * tfem_cg_iteration; levels / n_levels / coarse_inv / n_coarse as in tfem_amg_vcycle, and the    \
+   * finest level (or the coarse operator when n_levels == 0) must have n rows. */                  \
+  int tfem_pcg_iteration_##SUF(int64_t n, const int32_t* crow, const int32_t* col, const T* val,   \
+                               const uint8_t* keep, const tfem_amg_level* host_levels,             \
+                               int32_t n_levels, const T* coarse_inv, int64_t n_coarse, T* x,      \
+                               T* r, T* z, T* p, T* ap, T* partial, int32_t n_partial, T* scal,    \
+                               void* stream);                                                      \
+  /* One symmetric AMG V-cycle z = M_AMG r from a zero initial guess: on every level x = w D^-1 b,  \
+   * b_c = R (b - A x), recursion, x += P e_c, y = x + w D^-1 (b - A x); the coarsest system is     \
+   * solved by the dense inverse coarse_inv [n_coarse, n_coarse] (row-major, 1 <= n_coarse <=       \
+   * 32768), one warp per row.  host_levels: HOST array of n_levels >= 0 levels, finest first (the   \
+   * pointers inside are device memory; their work vectors are overwritten).  r, z [levels[0].n].   \
+   * Fixed-order sums, no allocation, no synchronisation: bitwise reproducible and graph-capturable. \
+   * TFEM_ERR_BAD_ARG for a NULL pointer or sizes that do not chain (levels[l].n_coarse ==           \
+   * levels[l+1].n, last == n_coarse). */                                                          \
+  int tfem_amg_vcycle_##SUF(const tfem_amg_level* host_levels, int32_t n_levels,                   \
+                            const T* coarse_inv, int64_t n_coarse, const T* r, T* z,              \
+                            void* stream);                                                         \
+  /* AMG set-up, strength of connection: diag [n] = a_ii (0 when the row stores none) and, per       \
+   * stored entry, strong [nnz] = 1 when j != i and |a_ij| >= theta sqrt(|a_ii a_jj|), else 0.       \
+   * theta >= 0. */                                                                                \
+  int tfem_amg_strength_##SUF(int64_t n, const int32_t* crow, const int32_t* col, const T* val,    \
+                              double theta, T* diag, uint8_t* strong, void* stream);              \
+  /* Deterministic SpGEMM C = op(A) B by expansion, stable radix sort of the 64-bit (row, col) keys, \
+   * run-length encoding and in-order segmented sums (bitwise reproducible, no float atomics).       \
+   * A [n_rows_a x .] CSR; transpose = 1 takes op(A) = A^T; b_crow == NULL stands for B = I (so      \
+   * transpose = 1 with no B is the transpose of A).  n_rows_c / n_cols_c: shape of C.  n_products  \
+   * must be the exact number of products: sum over the entries (i, k) of A of the length of row k   \
+   * of B (row i with transpose; 1 without B).  Outputs sized for the worst case: c_crow            \
+   * [n_rows_c + 1], c_col / c_val [n_products] (the first *c_nnz valid), c_nnz DEVICE int64.       \
+   * workspace: at least tfem_csr_spgemm_workspace(n_rows_a, n_products) bytes. */                  \
+  int tfem_csr_spgemm_##SUF(int64_t n_rows_a, const int32_t* a_crow, const int32_t* a_col,         \
+                            const T* a_val, int transpose, const int32_t* b_crow,                 \
+                            const int32_t* b_col, const T* b_val, int64_t n_rows_c,               \
+                            int64_t n_cols_c, int64_t n_products, void* workspace,                \
+                            int64_t workspace_bytes, int32_t* c_crow, int32_t* c_col, T* c_val,   \
+                            int64_t* c_nnz, void* stream);                                         \
   /* SURVEY.md 8(f).3 -- fused MLP-at-quadrature-points producer: N(x) and dN/dx of the body of the\
    * reference's FeedForwardNeuralNetwork (model/neural_network.py:50-100: Linear(d,w) act         \
    * {Linear(w,w) act} x n_square Linear(w,1)) by forward-mode differentiation in one pass over    \
@@ -355,6 +419,24 @@ int tfem_csr_symbolic_workspace(int64_t n_el, int64_t n_dof, int64_t* bytes);
 int tfem_csr_symbolic(int64_t n_el, const int32_t* dof_conn, int64_t n_dof, void* workspace, int64_t workspace_bytes,
                       int32_t* crow, int32_t* col, int32_t* seg, int32_t* perm, int32_t* lin_seg, int32_t* lin_perm,
                       int64_t* keys, int64_t* nnz, void* stream);
+
+/* AMG set-up, aggregation by parallel MIS(2) (Bell, Dalton, Olson 2012) on the strength graph (strong [nnz] from
+ * tfem_amg_strength).  key [n] (uint64) = state << 61 | (hash32(i, level) >> 3) << 32 | i, state 0 = out,
+ * 1 = undecided, 2 = in (a root); nodes without a strong connection start out.
+ * tfem_amg_mis2_round: one round (init != 0 first writes the initial keys): two sweeps t = max(t, max over strong
+ *   neighbours) from key into scratch [2n] (each sweep reads one buffer and writes the other), then an undecided node
+ *   whose own key is the maximum becomes in and one whose maximum is an in node becomes out.  *n_undecided (DEVICE
+ *   int32) = nodes still undecided; the caller repeats rounds until it reads 0 (each round decides at least one).
+ * tfem_amg_aggregate: after the last round, agg [n] (int32) = rank of the node's root among the roots for every root
+ *   and for each node with a strong root neighbour (the one of the largest key), else the aggregate of its strong
+ *   neighbour of the largest key among those so assigned, -1 for nodes without a strong connection; *n_agg (DEVICE
+ *   int32) = number of roots.  workspace: at least tfem_amg_aggregate_workspace() bytes. */
+int tfem_amg_mis2_round(int64_t n, const int32_t* crow, const int32_t* col, const uint8_t* strong, int32_t level, int init,
+                        uint64_t* key, uint64_t* scratch, int32_t* n_undecided, void* stream);
+int tfem_amg_aggregate_workspace(int64_t n, int64_t* bytes);
+int tfem_amg_aggregate(int64_t n, const int32_t* crow, const int32_t* col, const uint8_t* strong, const uint64_t* key,
+                       void* workspace, int64_t workspace_bytes, int32_t* agg, int32_t* n_agg, void* stream);
+int tfem_csr_spgemm_workspace(int64_t n_rows_a, int64_t n_products, int64_t* bytes);
 
 /* SURVEY 8(f).2 -- edge topology on the device, replacing AbstractMesh._compute_interior_and_boundary_edges /
  * _compute_cells_4_edges (mesh/abstract_mesh.py:104-255, mesh/meshes_tri.py:54-123).

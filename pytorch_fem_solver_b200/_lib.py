@@ -40,6 +40,15 @@ class Bilinear(Structure):
     _fields_ = [("alpha", c_double), ("beta", c_double)]
 
 
+class AmgLevel(Structure):
+    """struct tfem_amg_level."""
+
+    _fields_ = [("n", c_int64), ("n_coarse", c_int64)] + [
+        (name, c_void_p)
+        for name in ("a_crow", "a_col", "a_val", "p_crow", "p_col", "p_val", "r_crow", "r_col", "r_val", "wdinv", "x", "rc", "ec")
+    ]
+
+
 class TilePlan(Structure):
     """struct tfem_tile_plan."""
 
@@ -88,6 +97,10 @@ _TYPED = {
     "tfem_edge_jump": [I64, c_int, c_int, P, P, P, P, P, P],
     "tfem_csr_spmv": [I64, P, P, P, P, P, P, P],
     "tfem_cg_iteration": [I64, P, P, P, P, P, P, P, P, P, P, P, c_int32, P, P],
+    "tfem_pcg_iteration": [I64, P, P, P, P, POINTER(AmgLevel), c_int32, P, I64, P, P, P, P, P, P, c_int32, P, P],
+    "tfem_amg_vcycle": [POINTER(AmgLevel), c_int32, P, I64, P, P, P],
+    "tfem_amg_strength": [I64, P, P, P, c_double, P, P, P],
+    "tfem_csr_spgemm": [I64, P, P, P, c_int, P, P, P, I64, I64, I64, P, I64, P, P, P, P, P],
     "tfem_mlp_value_grad": [I64, c_int, c_int, c_int, c_int, P, P, P, P, P],
     "tfem_mlp_value_grad_bwd": [I64, c_int, c_int, c_int, c_int, P, P, P, P, P, c_int, P, P],
     "tfem_iface_pack": [I64, P, P, P, P],
@@ -98,6 +111,10 @@ _UNTYPED = {
     "tfem_coo_keys": ([I64, P, I64, P, P], c_int),
     "tfem_csr_symbolic_workspace": ([I64, I64, POINTER(c_int64)], c_int),
     "tfem_csr_symbolic": ([I64, P, I64, P, I64, P, P, P, P, P, P, P, P, P], c_int),
+    "tfem_amg_mis2_round": ([I64, P, P, P, c_int32, c_int, P, P, P, P], c_int),
+    "tfem_amg_aggregate_workspace": ([I64, POINTER(c_int64)], c_int),
+    "tfem_amg_aggregate": ([I64, P, P, P, P, P, I64, P, P, P], c_int),
+    "tfem_csr_spgemm_workspace": ([I64, I64, POINTER(c_int64)], c_int),
     "tfem_half_edges_workspace": ([I64, I64, POINTER(c_int64)], c_int),
     "tfem_half_edges": ([I64, I64, I64, P, POINTER(c_int32), P, I64, P, P, P, P, P, P], c_int),
     "tfem_edge_cells": ([I64, I64, I64, P, c_int, P, P, I64, P, P, P], c_int),

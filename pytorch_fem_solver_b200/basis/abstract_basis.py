@@ -428,14 +428,22 @@ class AbstractBasis(abc.ABC):
         """Zero vector of shape (nb_dofs, 1) (reference :173-175)."""
         return torch.zeros(self._basis_parameters["linear_form_shape"], dtype=self.dtype, device=self.device)
 
+    def inner_dofs_mask(self) -> torch.Tensor:
+        """uint8 [nb_dofs]: 1 on the inner DOFs -- the keep mask of the CSR solve (build `sparse.amg` with it)."""
+        keep = torch.zeros(self._basis_parameters["linear_form_shape"][0], dtype=torch.uint8, device=self.device)
+        keep[self._basis_parameters["inner_dofs"]] = 1
+        return keep
+
     def solve(self, matrix: torch.Tensor, solution: torch.Tensor, vector: torch.Tensor, only_inner_dofs: bool = True,
-              rtol: float = 1e-10, max_iterations=None):
+              rtol: float = 1e-10, max_iterations=None, preconditioner=None):
         """Solve the (reduced) system and add the result to `solution` (reference :177-195).
 
         Dense matrices take the reference's direct solve.  A CSR matrix too large to densify
         (more than DENSE_LIMIT unknowns) is solved by preconditioned conjugate gradients on the
         CSR arrays (`sparse.cg`, symmetric positive definite systems such as stiffness / mass);
-        the run's `sparse.CgInfo` is kept in `self.last_solve_info`."""
+        the run's `sparse.CgInfo` is kept in `self.last_solve_info`.  `preconditioner`: on that path, a
+        `sparse.amg(matrix, self.inner_dofs_mask())` hierarchy (built with keep=None when
+        only_inner_dofs is False) replaces Jacobi; the direct solve ignores it."""
         inner = self._basis_parameters["inner_dofs"]
         if matrix.layout == torch.sparse_csr and matrix.shape[-1] > DENSE_LIMIT:
             from .. import sparse
@@ -445,7 +453,7 @@ class AbstractBasis(abc.ABC):
                 keep = torch.zeros(matrix.shape[-1], dtype=torch.uint8, device=matrix.device)
                 keep[inner] = 1
             x, info = sparse.cg(matrix.crow_indices().to(torch.int32), matrix.col_indices().to(torch.int32), matrix.values(),
-                                vector, keep, rtol=rtol, max_iterations=max_iterations)
+                                vector, keep, rtol=rtol, max_iterations=max_iterations, preconditioner=preconditioner)
             self.last_solve_info = info
             if not info.converged:
                 raise RuntimeError(f"conjugate gradients stopped at relative residual {info.relative_residual:.3e} "

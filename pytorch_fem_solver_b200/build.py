@@ -19,7 +19,7 @@ CSRC = os.path.join(PKG, "csrc")
 LIB_DIR = os.path.join(PKG, "lib")
 LIB_PATH = os.path.join(LIB_DIR, "libtfem_b200.so")
 STAMP = os.path.join(LIB_DIR, "libtfem_b200.stamp")
-SOURCES = ["geometry.cu", "forms.cu", "scatter.cu", "interp.cu", "sparse.cu", "symbolic.cu", "topology.cu", "mlp.cu", "assemble_tiled.cu"]
+SOURCES = ["geometry.cu", "forms.cu", "scatter.cu", "interp.cu", "sparse.cu", "symbolic.cu", "topology.cu", "mlp.cu", "assemble_tiled.cu", "amg.cu"]
 NVCC_FLAGS = [
     "-O3",
     "-std=c++17",

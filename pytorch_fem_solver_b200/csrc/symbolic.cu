@@ -146,3 +146,201 @@ extern "C" int tfem_csr_symbolic(int64_t n_el, const int32_t* dof_conn, int64_t 
   lower_bound_kernel<int32_t><<<blocks_for(n_dof + 1, 256), 256, 0, s>>>(form_sorted, nullptr, n3, n_dof, 1, lin_seg);
   return check_launch();
 }
+
+// ---------------------------------------------------------------------------------------------
+// Deterministic expand-sort-reduce SpGEMM C = op(A) B (AMG set-up: P = S T, A P, R = P^T, R (A P)).
+// Every product a_ik b_kj is written with its 64-bit key row * n_cols_c + col; a stable radix sort of the keys
+// (only the bits a key can have) with the product index as payload, run-length encoding and a prefix sum give
+// the CSR pattern, and tfem_scatter_bilinear sums each run left to right -- in product order, so C is bitwise
+// reproducible with no float atomics.  op(A) = A^T takes the products of A entry (i, k) with row i of B, keyed
+// (k, j); B == NULL stands for the identity (the transpose is then the same program on swapped keys).
+// ---------------------------------------------------------------------------------------------
+extern "C" int tfem_scatter_bilinear_f64(int64_t nnz, const int32_t* seg, const int32_t* perm, const double* local, double* csr_val,
+                                         void* stream);
+extern "C" int tfem_scatter_bilinear_f32(int64_t nnz, const int32_t* seg, const int32_t* perm, const float* local, float* csr_val,
+                                         void* stream);
+
+namespace tfem {
+
+inline int scatter_bilinear(int64_t n, const int32_t* seg, const int32_t* perm, const double* v, double* out, void* s) {
+  return tfem_scatter_bilinear_f64(n, seg, perm, v, out, s);
+}
+inline int scatter_bilinear(int64_t n, const int32_t* seg, const int32_t* perm, const float* v, float* out, void* s) {
+  return tfem_scatter_bilinear_f32(n, seg, perm, v, out, s);
+}
+
+// products of row i of op(A): sum over its entries of the length of the B row they meet (1 without B)
+__global__ void spgemm_count_kernel(int n_rows_a, const int32_t* __restrict__ a_crow, const int32_t* __restrict__ a_col, int transpose,
+                                    const int32_t* __restrict__ b_crow, int32_t* __restrict__ counts) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i > n_rows_a) return;
+  if (i == n_rows_a) {
+    counts[i] = 0;
+    return;
+  }
+  const int begin = a_crow[i], end = a_crow[i + 1];
+  int c = end - begin;
+  if (b_crow != nullptr) {
+    if (transpose) {
+      c *= b_crow[i + 1] - b_crow[i];
+    } else {
+      c = 0;
+      for (int k = begin; k < end; ++k) c += b_crow[a_col[k] + 1] - b_crow[a_col[k]];
+    }
+  }
+  counts[i] = c;
+}
+
+template <typename T>
+__global__ void spgemm_expand_kernel(int n_rows_a, const int32_t* __restrict__ a_crow, const int32_t* __restrict__ a_col,
+                                     const T* __restrict__ a_val, int transpose, const int32_t* __restrict__ b_crow,
+                                     const int32_t* __restrict__ b_col, const T* __restrict__ b_val, int64_t n_cols_c,
+                                     const int32_t* __restrict__ offset, int64_t capacity, int64_t* __restrict__ keys,
+                                     int32_t* __restrict__ index, T* __restrict__ prod) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n_rows_a) return;
+  int64_t at = offset[i];
+  for (int k = a_crow[i]; k < a_crow[i + 1]; ++k) {
+    const int j = a_col[k];
+    const T a = a_val[k];
+    const int64_t row = transpose ? j : i;
+    if (b_crow == nullptr) {
+      if (at < capacity) {
+        keys[at] = row * n_cols_c + (transpose ? i : j);
+        index[at] = (int32_t)at;
+        prod[at] = a;
+      }
+      ++at;
+      continue;
+    }
+    const int brow = transpose ? i : j;
+    for (int q = b_crow[brow]; q < b_crow[brow + 1]; ++q, ++at) {
+      if (at >= capacity) continue;
+      keys[at] = row * n_cols_c + b_col[q];
+      index[at] = (int32_t)at;
+      prod[at] = a * b_val[q];
+    }
+  }
+}
+
+struct SpgemmLayout {
+  size_t counts, offset, keys_in, keys_sorted, index, perm, prod, runs, seg, unique, cub_temp, cub_bytes, total;
+};
+
+inline int spgemm_layout(int64_t n_rows_a, int64_t n_products, SpgemmLayout* out) {
+  size_t sort = 0, rle = 0, scan_rows = 0, scan_runs = 0;
+  if (cub::DeviceRadixSort::SortPairs(nullptr, sort, (const int64_t*)nullptr, (int64_t*)nullptr, (const int32_t*)nullptr, (int32_t*)nullptr,
+                                      (int)n_products) != cudaSuccess)
+    return TFEM_ERR_LAUNCH;
+  if (cub::DeviceRunLengthEncode::Encode(nullptr, rle, (const int64_t*)nullptr, (int64_t*)nullptr, (int32_t*)nullptr, (int64_t*)nullptr,
+                                         (int)n_products) != cudaSuccess)
+    return TFEM_ERR_LAUNCH;
+  if (cub::DeviceScan::ExclusiveSum(nullptr, scan_rows, (const int32_t*)nullptr, (int32_t*)nullptr, (int)(n_rows_a + 1)) != cudaSuccess)
+    return TFEM_ERR_LAUNCH;
+  if (cub::DeviceScan::ExclusiveSum(nullptr, scan_runs, (const int32_t*)nullptr, (int32_t*)nullptr, (int)(n_products + 1)) != cudaSuccess)
+    return TFEM_ERR_LAUNCH;
+  size_t cub_bytes = sort;
+  cub_bytes = rle > cub_bytes ? rle : cub_bytes;
+  cub_bytes = scan_rows > cub_bytes ? scan_rows : cub_bytes;
+  cub_bytes = scan_runs > cub_bytes ? scan_runs : cub_bytes;
+  const size_t np = (size_t)n_products;
+  size_t at = 0;
+  out->counts = at;      at += align256(4 * (size_t)(n_rows_a + 1));
+  out->offset = at;      at += align256(4 * (size_t)(n_rows_a + 1));
+  out->keys_in = at;     at += align256(8 * np);
+  out->keys_sorted = at; at += align256(8 * np);
+  out->index = at;       at += align256(4 * np);
+  out->perm = at;        at += align256(4 * np);
+  out->prod = at;        at += align256(8 * np);  // sized for fp64 products
+  out->runs = at;        at += align256(4 * (np + 1));
+  out->seg = at;         at += align256(4 * (np + 1));
+  out->unique = at;      at += align256(8 * np);
+  out->cub_temp = at;    at += align256(cub_bytes);
+  out->cub_bytes = cub_bytes;
+  out->total = at;
+  return TFEM_OK;
+}
+
+template <typename T>
+int csr_spgemm(int64_t n_rows_a, const int32_t* a_crow, const int32_t* a_col, const T* a_val, int transpose, const int32_t* b_crow,
+               const int32_t* b_col, const T* b_val, int64_t n_rows_c, int64_t n_cols_c, int64_t n_products, void* workspace,
+               int64_t workspace_bytes, int32_t* c_crow, int32_t* c_col, T* c_val, int64_t* c_nnz, void* stream) {
+  if (n_rows_a < 0 || n_rows_c < 0 || n_cols_c <= 0 || n_products < 0 || (transpose != 0 && transpose != 1)) return TFEM_ERR_BAD_ARG;
+  if (!a_crow || !workspace || !c_crow || !c_nnz) return TFEM_ERR_BAD_ARG;
+  if ((n_products > 0 || n_rows_a > 0) && (!a_col || !a_val)) return TFEM_ERR_BAD_ARG;
+  if (b_crow != nullptr && (!b_col || !b_val)) return TFEM_ERR_BAD_ARG;
+  if (n_products > 0 && (!c_col || !c_val)) return TFEM_ERR_BAD_ARG;
+  if (n_rows_a >= kMaxIndex || n_rows_c >= kMaxIndex || n_cols_c >= kMaxIndex || n_products >= kMaxIndex) return TFEM_ERR_TOO_LARGE;
+  SpgemmLayout lay{};
+  int status = spgemm_layout(n_rows_a, n_products > 0 ? n_products : 1, &lay);
+  if (status != TFEM_OK) return status;
+  if ((size_t)workspace_bytes < lay.total) return TFEM_ERR_BAD_ARG;
+  auto s = static_cast<cudaStream_t>(stream);
+  if (n_products == 0) {
+    if (cudaMemsetAsync(c_crow, 0, 4 * (size_t)(n_rows_c + 1), s) != cudaSuccess) return TFEM_ERR_LAUNCH;
+    if (cudaMemsetAsync(c_nnz, 0, sizeof(int64_t), s) != cudaSuccess) return TFEM_ERR_LAUNCH;
+    return check_launch();
+  }
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  int32_t* counts = reinterpret_cast<int32_t*>(ws + lay.counts);
+  int32_t* offset = reinterpret_cast<int32_t*>(ws + lay.offset);
+  int64_t* keys_in = reinterpret_cast<int64_t*>(ws + lay.keys_in);
+  int64_t* keys_sorted = reinterpret_cast<int64_t*>(ws + lay.keys_sorted);
+  int32_t* index = reinterpret_cast<int32_t*>(ws + lay.index);
+  int32_t* perm = reinterpret_cast<int32_t*>(ws + lay.perm);
+  T* prod = reinterpret_cast<T*>(ws + lay.prod);
+  int32_t* runs = reinterpret_cast<int32_t*>(ws + lay.runs);
+  int32_t* seg = reinterpret_cast<int32_t*>(ws + lay.seg);
+  int64_t* unique = reinterpret_cast<int64_t*>(ws + lay.unique);
+  void* cub_temp = ws + lay.cub_temp;
+  size_t cub_bytes = lay.cub_bytes;
+
+  spgemm_count_kernel<<<blocks_for(n_rows_a + 1, 256), 256, 0, s>>>((int)n_rows_a, a_crow, a_col, transpose, b_crow, counts);
+  if (cub::DeviceScan::ExclusiveSum(cub_temp, cub_bytes, counts, offset, (int)(n_rows_a + 1), s) != cudaSuccess) return TFEM_ERR_LAUNCH;
+  spgemm_expand_kernel<T><<<blocks_for(n_rows_a, 256), 256, 0, s>>>((int)n_rows_a, a_crow, a_col, a_val, transpose, b_crow, b_col, b_val,
+                                                                     n_cols_c, offset, n_products, keys_in, index, prod);
+  cub_bytes = lay.cub_bytes;
+  if (cub::DeviceRadixSort::SortPairs(cub_temp, cub_bytes, keys_in, keys_sorted, index, perm, (int)n_products, 0,
+                                      bits_for(n_rows_c * n_cols_c), s) != cudaSuccess)
+    return TFEM_ERR_LAUNCH;
+  if (cudaMemsetAsync(runs, 0, 4 * (size_t)(n_products + 1), s) != cudaSuccess) return TFEM_ERR_LAUNCH;
+  cub_bytes = lay.cub_bytes;
+  if (cub::DeviceRunLengthEncode::Encode(cub_temp, cub_bytes, keys_sorted, unique, runs, c_nnz, (int)n_products, s) != cudaSuccess)
+    return TFEM_ERR_LAUNCH;
+  cub_bytes = lay.cub_bytes;
+  // seg[p] = first sorted product of entry p; entries past nnz have empty runs and sum to zero
+  if (cub::DeviceScan::ExclusiveSum(cub_temp, cub_bytes, runs, seg, (int)(n_products + 1), s) != cudaSuccess) return TFEM_ERR_LAUNCH;
+  status = scatter_bilinear(n_products, seg, perm, prod, c_val, stream);
+  if (status != TFEM_OK) return status;
+  split_keys_kernel<<<blocks_for(n_products + 1, 256), 256, 0, s>>>(unique, c_nnz, n_cols_c, n_products, c_col, seg);
+  lower_bound_kernel<int64_t><<<blocks_for(n_rows_c + 1, 256), 256, 0, s>>>(unique, c_nnz, 0, n_rows_c, n_cols_c, c_crow);
+  return check_launch();
+}
+
+}  // namespace tfem
+
+extern "C" int tfem_csr_spgemm_workspace(int64_t n_rows_a, int64_t n_products, int64_t* bytes) {
+  if (n_rows_a < 0 || n_products < 0 || !bytes) return TFEM_ERR_BAD_ARG;
+  if (n_rows_a >= tfem::kMaxIndex || n_products >= tfem::kMaxIndex) return TFEM_ERR_TOO_LARGE;
+  tfem::SpgemmLayout lay{};
+  const int status = tfem::spgemm_layout(n_rows_a, n_products > 0 ? n_products : 1, &lay);
+  if (status != TFEM_OK) return status;
+  *bytes = (int64_t)lay.total;
+  return TFEM_OK;
+}
+
+extern "C" int tfem_csr_spgemm_f64(int64_t n_rows_a, const int32_t* a_crow, const int32_t* a_col, const double* a_val, int transpose,
+                                   const int32_t* b_crow, const int32_t* b_col, const double* b_val, int64_t n_rows_c, int64_t n_cols_c,
+                                   int64_t n_products, void* workspace, int64_t workspace_bytes, int32_t* c_crow, int32_t* c_col,
+                                   double* c_val, int64_t* c_nnz, void* stream) {
+  return tfem::csr_spgemm<double>(n_rows_a, a_crow, a_col, a_val, transpose, b_crow, b_col, b_val, n_rows_c, n_cols_c, n_products, workspace,
+                                  workspace_bytes, c_crow, c_col, c_val, c_nnz, stream);
+}
+
+extern "C" int tfem_csr_spgemm_f32(int64_t n_rows_a, const int32_t* a_crow, const int32_t* a_col, const float* a_val, int transpose,
+                                   const int32_t* b_crow, const int32_t* b_col, const float* b_val, int64_t n_rows_c, int64_t n_cols_c,
+                                   int64_t n_products, void* workspace, int64_t workspace_bytes, int32_t* c_crow, int32_t* c_col,
+                                   float* c_val, int64_t* c_nnz, void* stream) {
+  return tfem::csr_spgemm<float>(n_rows_a, a_crow, a_col, a_val, transpose, b_crow, b_col, b_val, n_rows_c, n_cols_c, n_products, workspace,
+                                 workspace_bytes, c_crow, c_col, c_val, c_nnz, stream);
+}

@@ -263,6 +263,114 @@ def cg_iteration_raw(crow: Tensor, col: Tensor, val: Tensor, keep: Optional[Tens
 
 
 # ------------------------------------------------------------------------------------------------
+# smoothed-aggregation AMG (set-up and V-cycle; sparse.amg builds the hierarchy)
+# ------------------------------------------------------------------------------------------------
+
+
+def amg_strength(crow: Tensor, col: Tensor, val: Tensor, theta: float) -> Tuple[Tensor, Tensor]:
+    """(diag [n], strong [nnz] uint8): strength of connection |a_ij| >= theta sqrt(|a_ii a_jj|), i != j."""
+    device = check_cuda(crow, col, val)
+    n = crow.shape[0] - 1
+    diag = torch.empty(n, dtype=val.dtype, device=device)
+    strong = torch.empty(col.shape[0], dtype=torch.uint8, device=device)
+    call("tfem_amg_strength", val.dtype, device, n, ptr(crow), ptr(col), ptr(val), float(theta), ptr(diag), ptr(strong))
+    return diag, strong
+
+
+def _workspace(name: str, *sizes) -> int:
+    import ctypes
+
+    need = ctypes.c_int64(0)
+    status = getattr(_lib.load(), name)(*sizes, ctypes.byref(need))
+    if status != 0:
+        raise TfemError(f"{name} failed ({status})")
+    return int(need.value)
+
+
+def amg_aggregate(crow: Tensor, col: Tensor, strong: Tensor, level: int) -> Tuple[Tensor, int]:
+    """(agg [n] int32, n_agg): parallel MIS(2) aggregation of the strength graph (-1: no strong connection).
+    Set-up: the host reads the undecided count after every round."""
+    device = check_cuda(crow, col, strong)
+    n = crow.shape[0] - 1
+    key = torch.empty(n, dtype=torch.int64, device=device)
+    scratch = torch.empty(2 * n, dtype=torch.int64, device=device)
+    counter = torch.zeros(1, dtype=torch.int32, device=device)
+    for round_ in range(n + 1):  # every round decides at least the undecided node of the largest key
+        call("tfem_amg_mis2_round", None, device, n, ptr(crow), ptr(col), ptr(strong), level, int(round_ == 0), ptr(key), ptr(scratch),
+                    ptr(counter))
+        if int(counter.item()) == 0:
+            break
+    else:
+        raise TfemError("MIS(2) aggregation did not terminate")
+    workspace = torch.empty(_workspace("tfem_amg_aggregate_workspace", n), dtype=torch.uint8, device=device)
+    agg = torch.empty(n, dtype=torch.int32, device=device)
+    call("tfem_amg_aggregate", None, device, n, ptr(crow), ptr(col), ptr(strong), ptr(key), ptr(workspace), workspace.numel(),
+                ptr(agg), ptr(counter))
+    return agg, int(counter.item())
+
+
+def csr_spgemm(a: Tuple[Tensor, Tensor, Tensor], n_cols_a: int, b: Optional[Tuple[Tensor, Tensor, Tensor]] = None,
+               n_cols_b: int = 0, transpose: bool = False) -> Tuple[Tensor, Tensor, Tensor]:
+    """C = op(A) B as CSR (crow, col, val), op(A) = A^T with `transpose`, B = identity when None (tfem_csr_spgemm)."""
+    a_crow, a_col, a_val = a
+    device = check_cuda(a_crow, a_col, a_val, *(b or ()))
+    n_rows_a = a_crow.shape[0] - 1
+    n_rows_c = n_cols_a if transpose else n_rows_a
+    n_cols_c = (n_rows_a if transpose else n_cols_a) if b is None else n_cols_b
+    a_len = (a_crow[1:] - a_crow[:-1]).long()
+    if b is None:
+        n_products = a_col.shape[0]
+    else:
+        b_len = (b[0][1:] - b[0][:-1]).long()
+        n_products = int((a_len * b_len).sum()) if transpose else int(b_len[a_col.long()].sum())
+    workspace = torch.empty(_workspace("tfem_csr_spgemm_workspace", n_rows_a, n_products), dtype=torch.uint8, device=device)
+    c_crow = torch.empty(n_rows_c + 1, dtype=torch.int32, device=device)
+    c_col = torch.empty(max(n_products, 1), dtype=torch.int32, device=device)
+    c_val = torch.empty(max(n_products, 1), dtype=a_val.dtype, device=device)
+    c_nnz = torch.zeros(1, dtype=torch.int64, device=device)
+    b_crow, b_col, b_val = b if b is not None else (None, None, None)
+    call("tfem_csr_spgemm", a_val.dtype, device, n_rows_a, ptr(a_crow), ptr(a_col), ptr(a_val), int(transpose), ptr(b_crow), ptr(b_col),
+         ptr(b_val), n_rows_c, max(n_cols_c, 1), n_products, ptr(workspace), workspace.numel(), ptr(c_crow), ptr(c_col), ptr(c_val),
+         ptr(c_nnz))
+    nnz = int(c_nnz.item())
+    return c_crow, c_col[:nnz].clone(), c_val[:nnz].clone()
+
+
+def amg_levels_struct(hierarchy):
+    """ctypes array of struct tfem_amg_level over the device tensors of an `sparse.AmgHierarchy` (kept alive by it)."""
+    levels = hierarchy.levels
+    array = (_lib.AmgLevel * max(len(levels), 1))()
+    for slot, lev in zip(array, levels):
+        slot.n, slot.n_coarse = lev.n, lev.n_coarse
+        for name in ("a_crow", "a_col", "a_val", "p_crow", "p_col", "p_val", "r_crow", "r_col", "r_val", "wdinv", "x", "rc", "ec"):
+            setattr(slot, name, ptr(getattr(lev, name)))
+    return array
+
+
+def amg_vcycle_raw(hierarchy, r: Tensor, z: Tensor) -> None:
+    """z = M_AMG r (one V-cycle, tfem_amg_vcycle) into a preallocated vector; CUDA-graph capturable."""
+    device = check_cuda(r, z, hierarchy.coarse_inv)
+    call("tfem_amg_vcycle", r.dtype, device, hierarchy.struct, len(hierarchy.levels), ptr(hierarchy.coarse_inv),
+         hierarchy.coarse_inv.shape[0], ptr(r), ptr(z))
+
+
+def amg_vcycle(hierarchy, r: Tensor) -> Tensor:
+    """z = M_AMG r."""
+    z = torch.empty_like(r)
+    amg_vcycle_raw(hierarchy, r, z)
+    return z
+
+
+def pcg_iteration_raw(crow: Tensor, col: Tensor, val: Tensor, keep: Optional[Tensor], hierarchy, x: Tensor, r: Tensor, z: Tensor,
+                      p: Tensor, ap: Tensor, partial: Tensor, scal: Tensor) -> None:
+    """One AMG-preconditioned CG iteration on preallocated state (see tfem_pcg_iteration); CUDA-graph capturable."""
+    device = check_cuda(crow, col, val, x, r, z, p, ap, partial, scal, hierarchy.coarse_inv)
+    call("tfem_pcg_iteration", val.dtype, device, crow.shape[0] - 1, ptr(crow), ptr(col), ptr(val),
+         ptr(keep) if keep is not None else None, hierarchy.struct, len(hierarchy.levels), ptr(hierarchy.coarse_inv),
+         hierarchy.coarse_inv.shape[0], ptr(x), ptr(r), ptr(z), ptr(p), ptr(ap), ptr(partial), partial.shape[0] // 2, ptr(scal))
+
+
+# ------------------------------------------------------------------------------------------------
 # fused named forms
 # ------------------------------------------------------------------------------------------------
 

@@ -7,12 +7,16 @@ conjugate gradients on the full-length vectors with the non-interior rows and co
 one iteration is three hand-written kernels (`tfem_cg_iteration`: SpMV + p.Ap, the vector updates
 + r.z, the new direction) with every dot product reduced in a fixed order and the scalars kept on
 the device; the host looks at the residual only every `check_every` iterations.
+
+`amg()` builds a smoothed-aggregation algebraic multigrid hierarchy once, on the device, and
+`preconditioner=` replaces Jacobi by one V-cycle of it per iteration (`tfem_pcg_iteration`); the
+Gram matrix of a training loop is fixed, so one hierarchy serves every step (DESIGN.md §8(f).1).
 """
 
 from __future__ import annotations
 
-from dataclasses import dataclass
-from typing import Optional
+from dataclasses import dataclass, field
+from typing import List, Optional
 
 import torch
 
@@ -46,16 +50,21 @@ def cg(
     x0: Optional[torch.Tensor] = None,
     rtol: float = 1e-10,
     max_iterations: Optional[int] = None,
-    check_every: int = 50,
+    check_every: Optional[int] = None,
     use_graph: bool = True,
     fused: bool = True,
+    preconditioner: Optional["AmgHierarchy"] = None,
 ):
     """Solve `(M A M) x = M rhs` for symmetric positive definite `M A M`, `M = diag(keep)`.
 
     crow/col int32, val/rhs float; keep bool/uint8 of length n or None (every row).  Returns
     `(x, CgInfo)`; x is zero where keep is 0.  On CUDA one iteration is captured in a CUDA graph
     and replayed (`use_graph=False` keeps the eager loop); `fused=False` uses torch vector
-    updates around `tfem_csr_spmv` instead of the three-kernel `tfem_cg_iteration`."""
+    updates around `tfem_csr_spmv` instead of the three-kernel `tfem_cg_iteration`.
+
+    `preconditioner`: an `amg()` hierarchy of this matrix and keep mask (ValueError otherwise) replaces Jacobi by one
+    V-cycle per iteration (`tfem_pcg_iteration`).  The residual is checked every `check_every` iterations: 50 with
+    Jacobi, every iteration with AMG (which needs tens of iterations, not thousands)."""
     n = crow.shape[0] - 1
     b = rhs.reshape(-1).to(device=val.device, dtype=val.dtype)
     if b.shape[0] != n:
@@ -64,13 +73,19 @@ def cg(
     if keep is not None:
         keep8 = keep.reshape(-1).to(device=val.device, dtype=torch.uint8).contiguous()
         b = b * keep8.to(val.dtype)
-    diag = csr_diagonal(crow, col, val)
-    inv_diag = torch.where(diag != 0, 1.0 / diag, torch.ones_like(diag))
+    if preconditioner is not None:
+        preconditioner.check(crow, val, keep8)
+        inv_diag = None
+    else:
+        diag = csr_diagonal(crow, col, val)
+        inv_diag = torch.where(diag != 0, 1.0 / diag, torch.ones_like(diag))
+    if check_every is None:
+        check_every = 50 if preconditioner is None else 1
     x = torch.zeros_like(b) if x0 is None else x0.reshape(-1).to(device=val.device, dtype=val.dtype).clone()
     if keep8 is not None:
         x = x * keep8.to(val.dtype)
     r = b - ops.csr_spmv(crow, col, val, x, keep8) if x0 is not None else b.clone()
-    z = r * inv_diag
+    z = r * inv_diag if preconditioner is None else ops.amg_vcycle(preconditioner, r)
     p = z.clone()
     ap = torch.empty_like(p)
     rz = torch.dot(r, z).reshape(1)
@@ -94,13 +109,27 @@ def cg(
         alpha = rz / torch.dot(p, ap).clamp_min(tiny)
         x.addcmul_(p, alpha)
         r.addcmul_(ap, alpha, value=-1.0)
-        torch.mul(r, inv_diag, out=z)
+        if preconditioner is None:
+            torch.mul(r, inv_diag, out=z)
+        elif val.is_cuda:
+            ops.amg_vcycle_raw(preconditioner, r, z)
+        else:
+            z.copy_(ops.amg_vcycle(preconditioner, r))
         rz_new = torch.dot(r, z).reshape(1)
         p.mul_(rz_new / rz.clamp_min(tiny)).add_(z)
         rz.copy_(rz_new)
 
     fused_step = getattr(ops, "cg_iteration_raw", None) if (val.is_cuda and fused) else None
-    if fused_step is not None:
+    if fused_step is not None and preconditioner is not None:
+        # five launch groups per iteration (tfem_pcg_iteration): SpMV + p.Ap | x, r updates | V-cycle | r.z | new direction
+        blocks = 8 * torch.cuda.get_device_properties(val.device).multi_processor_count
+        partial = torch.zeros(2 * blocks, dtype=val.dtype, device=val.device)
+        scal = torch.cat([rz, rz]).contiguous()
+
+        def iteration():  # noqa: F811
+            ops.pcg_iteration_raw(crow, col, val, keep8, preconditioner, x, r, z, p, ap, partial, scal)
+
+    elif fused_step is not None:
         # three launches per iteration (tfem_cg_iteration): SpMV + p.Ap | x, r, z updates + r.z | new direction
         blocks = 8 * torch.cuda.get_device_properties(val.device).multi_processor_count
         partial = torch.zeros(2 * blocks, dtype=val.dtype, device=val.device)
@@ -151,18 +180,218 @@ def cg(
     return x, CgInfo(iterations, rel, converged)
 
 
+# ------------------------------------------------------------------------------------------------
+# smoothed-aggregation AMG preconditioner
+# ------------------------------------------------------------------------------------------------
+
+POWER_ITERATIONS = 15
+POWER_SALT = 0x10000  # hash salt of the power-iteration start vector (+ level); oracle/amg_oracle.py uses the same
+MAX_DENSE_COARSE = 32768  # the coarsest operator is inverted densely (tfem_amg_vcycle's limit)
+
+
+@dataclass
+class AmgLevel:
+    """One smoothed level: operator A, prolongator P, restriction R = P^T (CSR), omega D^-1 and work vectors."""
+
+    n: int
+    n_coarse: int
+    a_crow: torch.Tensor
+    a_col: torch.Tensor
+    a_val: torch.Tensor
+    p_crow: torch.Tensor
+    p_col: torch.Tensor
+    p_val: torch.Tensor
+    r_crow: torch.Tensor
+    r_col: torch.Tensor
+    r_val: torch.Tensor
+    wdinv: torch.Tensor
+    agg: torch.Tensor
+    rho: float
+    omega: float
+    x: torch.Tensor = field(init=False)
+    rc: torch.Tensor = field(init=False)
+    ec: torch.Tensor = field(init=False)
+
+    def __post_init__(self):
+        self.x = torch.zeros_like(self.wdinv)
+        self.rc = self.wdinv.new_zeros(self.n_coarse)
+        self.ec = self.wdinv.new_zeros(self.n_coarse)
+
+
+@dataclass
+class AmgHierarchy:
+    """The hierarchy `amg()` builds for one matrix and keep mask; pass it as `preconditioner=`.
+
+    levels: the smoothed levels, finest first; coarse_inv: dense inverse of the coarsest operator."""
+
+    levels: List[AmgLevel]
+    coarse_inv: torch.Tensor
+    coarse_nnz: int
+    keep: torch.Tensor  # uint8 [n] (ones when built without a mask)
+    nnz: int
+    theta: float
+    _struct: object = field(default=None, repr=False)
+
+    @property
+    def n(self) -> int:
+        return self.levels[0].n if self.levels else self.coarse_inv.shape[0]
+
+    @property
+    def dtype(self) -> torch.dtype:
+        return self.coarse_inv.dtype
+
+    @property
+    def device(self) -> torch.device:
+        return self.coarse_inv.device
+
+    @property
+    def grid_sizes(self) -> List[int]:
+        return [lev.n for lev in self.levels] + [self.coarse_inv.shape[0]]
+
+    @property
+    def operator_complexity(self) -> float:
+        """Stored entries of every level's operator over those of the finest."""
+        total = sum(lev.a_col.shape[0] for lev in self.levels) + self.coarse_nnz
+        return total / (self.levels[0].a_col.shape[0] if self.levels else max(self.coarse_nnz, 1))
+
+    @property
+    def rho(self) -> List[float]:
+        return [lev.rho for lev in self.levels]
+
+    @property
+    def omega(self) -> List[float]:
+        return [lev.omega for lev in self.levels]
+
+    @property
+    def struct(self):
+        """The host array of struct tfem_amg_level the V-cycle entry points read."""
+        if self._struct is None:
+            self._struct = ops.amg_levels_struct(self)
+        return self._struct
+
+    def summary(self) -> str:
+        rows = ", ".join(f"{n}" for n in self.grid_sizes)
+        rho = ", ".join(f"{r:.4f}" for r in self.rho)
+        return (f"{len(self.grid_sizes)} levels (rows {rows}), operator complexity {self.operator_complexity:.3f}, "
+                f"theta {self.theta}, rho(D^-1 A) per level [{rho}]")
+
+    def check(self, crow: torch.Tensor, val: torch.Tensor, keep8: Optional[torch.Tensor]) -> None:
+        """ValueError unless this hierarchy was built for a matrix of this size, nnz, dtype and device and this keep mask."""
+        n = crow.shape[0] - 1
+        if n != self.n or val.shape[0] != self.nnz or val.dtype != self.dtype or val.device != self.device:
+            raise ValueError(f"the AMG hierarchy was built for a {self.n}-row {self.dtype} matrix with {self.nnz} entries on {self.device}, "
+                             f"not for this {n}-row {val.dtype} matrix with {val.shape[0]} entries on {val.device}")
+        keep = torch.ones(n, dtype=torch.uint8, device=val.device) if keep8 is None else keep8
+        if not torch.equal(keep, self.keep):
+            raise ValueError("the AMG hierarchy was built for another keep mask")
+
+
+def _hash32(i: torch.Tensor, salt: int) -> torch.Tensor:
+    """oracle/amg_oracle.py hash32 in int64 arithmetic (products wrap; the low 32 bits are exact)."""
+    m = 0xFFFFFFFF
+    h = (i * 0x9E3779B1 + (salt * 0x85EBCA77 + 0x165667B1)) & m
+    h = h ^ (h >> 16)
+    h = (h * 0x85EBCA6B) & m
+    h = h ^ (h >> 13)
+    h = (h * 0xC2B2AE35) & m
+    return h ^ (h >> 16)
+
+
+def _masked_operator(crow, col, val, keep8):
+    """(M A M) + (I - M): masked rows and columns dropped, their diagonals set to 1."""
+    if keep8 is None:
+        return crow, col, val.clone()
+    n = crow.shape[0] - 1
+    row = torch.repeat_interleave(torch.arange(n, device=col.device), (crow[1:] - crow[:-1]).long())
+    k = keep8 != 0
+    on_diag = row == col.long()
+    live = (k[row] & k[col.long()]) | on_diag
+    v = torch.where(on_diag & ~k[row], torch.ones_like(val), val)
+    counts = torch.bincount(row[live], minlength=n)
+    new_crow = torch.cat([counts.new_zeros(1), torch.cumsum(counts, 0)]).to(torch.int32)
+    return new_crow, col[live].contiguous(), v[live].contiguous()
+
+
+def _spectral_radius(crow, col, val, inv_diag, level: int) -> float:
+    """rho(D^-1 A) by power iteration from a hash-generated (reproducible) start vector."""
+    n = crow.shape[0] - 1
+    v = _hash32(torch.arange(n, device=val.device), POWER_SALT + level).to(val.dtype) / 4294967296.0 - 0.5
+    rho = None
+    for _ in range(POWER_ITERATIONS):
+        w = inv_diag * ops.csr_spmv(crow, col, val, v)
+        nw = torch.linalg.vector_norm(w)
+        rho = nw / torch.linalg.vector_norm(v)
+        v = w / nw
+    return float(rho)
+
+
+def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float = 0.08, max_coarse: int = 1000,
+        max_levels: int = 12) -> AmgHierarchy:
+    """Smoothed-aggregation AMG hierarchy of the operator `cg` solves, (M A M) + (I - M), M = diag(keep), for a
+    symmetric positive definite CSR `matrix`; one-time set-up on the device.
+
+    Per level: strength |a_ij| >= theta sqrt(|a_ii a_jj|); aggregates by parallel MIS(2); tentative prolongator
+    T = 1 / sqrt(|aggregate|) (nodes without strong connections stay unaggregated: the smoother alone handles them);
+    rho(D^-1 A) by 15 power iterations; P = (I - omega D^-1 A) T, omega = 4 / (3 rho); R = P^T; A_c = R A P by the
+    deterministic SpGEMM.  Coarsening stops at <= max_coarse rows or max_levels levels; the coarsest operator is
+    inverted densely.  The result is reproducible run to run."""
+    crow, col, val = matrix.crow_indices().to(torch.int32), matrix.col_indices().to(torch.int32), matrix.values()
+    n = crow.shape[0] - 1
+    keep8 = None if keep is None else keep.reshape(-1).to(device=val.device, dtype=torch.uint8).contiguous()
+    if keep8 is not None and keep8.shape[0] != n:
+        raise ValueError("keep mask length does not match the matrix")
+    a = _masked_operator(crow, col, val, keep8)
+    levels: List[AmgLevel] = []
+    while a[0].shape[0] - 1 > max_coarse and len(levels) + 1 < max_levels:
+        level = len(levels)
+        a_crow, a_col, a_val = a
+        n_l = a_crow.shape[0] - 1
+        diag, strong = ops.amg_strength(a_crow, a_col, a_val, theta)
+        agg, n_agg = ops.amg_aggregate(a_crow, a_col, strong, level)
+        if n_agg == 0 or n_agg >= n_l:
+            break  # nothing left to coarsen: this operator is the coarsest
+        live = agg >= 0
+        size = torch.bincount(agg[live].long(), minlength=n_agg)
+        t_crow = torch.cat([size.new_zeros(1), torch.cumsum(live.long(), 0)]).to(torch.int32)
+        t_col = agg[live].contiguous()
+        t_val = (1.0 / torch.sqrt(size[t_col.long()].to(a_val.dtype))).contiguous()
+        inv_diag = 1.0 / diag
+        rho = _spectral_radius(a_crow, a_col, a_val, inv_diag, level)
+        omega = 4.0 / (3.0 * rho)
+        wdinv = (omega / diag).contiguous()
+        row = torch.repeat_interleave(torch.arange(n_l, device=a_val.device), (a_crow[1:] - a_crow[:-1]).long())
+        s_val = ((row == a_col.long()).to(a_val.dtype) - wdinv[row] * a_val).contiguous()
+        p = ops.csr_spgemm((a_crow, a_col, s_val), n_l, (t_crow, t_col, t_val), n_agg)
+        r = ops.csr_spgemm(p, n_agg, transpose=True)
+        ap = ops.csr_spgemm(a, n_l, p, n_agg)
+        a_c = ops.csr_spgemm(r, n_l, ap, n_agg)
+        levels.append(AmgLevel(n_l, n_agg, a_crow, a_col, a_val, *p, *r, wdinv, agg, rho, omega))
+        a = a_c
+    a_crow, a_col, a_val = a
+    n_c = a_crow.shape[0] - 1
+    if n_c > MAX_DENSE_COARSE:
+        raise ValueError(f"coarsening stopped at {n_c} rows, more than the dense coarsest solve takes ({MAX_DENSE_COARSE}); "
+                         "raise max_levels or lower theta")
+    dense = torch.zeros((n_c, n_c), dtype=a_val.dtype, device=a_val.device)
+    dense[torch.repeat_interleave(torch.arange(n_c, device=a_val.device), (a_crow[1:] - a_crow[:-1]).long()), a_col.long()] = a_val
+    coarse_inv = torch.linalg.inv(dense).contiguous()
+    keep_all = torch.ones(n, dtype=torch.uint8, device=val.device) if keep8 is None else keep8.clone()
+    return AmgHierarchy(levels, coarse_inv, a_col.shape[0], keep_all, val.shape[0], theta)
+
+
 class _CgSolve(torch.autograd.Function):
     """x = (M A M)^-1 M b through `cg`, differentiable w.r.t. b: for symmetric A the adjoint is one more solve,
     b_bar = (M A M)^-1 M x_bar (the matrix is a constant of the optimisation, as the Gram matrix of
     examples/example_weak.py:84-86 is)."""
 
     @staticmethod
-    def forward(ctx, b, crow, col, val, keep, rtol, max_iterations):
-        x, info = cg(crow, col, val, b.detach(), keep, rtol=rtol, max_iterations=max_iterations)
+    def forward(ctx, b, crow, col, val, keep, rtol, max_iterations, preconditioner):
+        x, info = cg(crow, col, val, b.detach(), keep, rtol=rtol, max_iterations=max_iterations, preconditioner=preconditioner)
         if not info.converged:
             raise RuntimeError(f"conjugate gradients stopped at relative residual {info.relative_residual:.3e} after {info.iterations} iterations")
         ctx.save_for_backward(crow, col, val)
         ctx.keep, ctx.rtol, ctx.max_iterations, ctx.shape = keep, rtol, max_iterations, b.shape
+        ctx.preconditioner = preconditioner
         ctx.info = info
         return x.reshape(b.shape)
 
@@ -170,27 +399,29 @@ class _CgSolve(torch.autograd.Function):
     def backward(ctx, x_bar):
         crow, col, val = ctx.saved_tensors
         if not bool(x_bar.any()):
-            return torch.zeros(ctx.shape, dtype=x_bar.dtype, device=x_bar.device), None, None, None, None, None, None
-        b_bar, info = cg(crow, col, val, x_bar.detach(), ctx.keep, rtol=ctx.rtol, max_iterations=ctx.max_iterations)
+            return torch.zeros(ctx.shape, dtype=x_bar.dtype, device=x_bar.device), None, None, None, None, None, None, None
+        b_bar, info = cg(crow, col, val, x_bar.detach(), ctx.keep, rtol=ctx.rtol, max_iterations=ctx.max_iterations,
+                         preconditioner=ctx.preconditioner)
         if not info.converged:
             raise RuntimeError(f"adjoint conjugate gradients stopped at relative residual {info.relative_residual:.3e}")
-        return b_bar.reshape(ctx.shape), None, None, None, None, None, None
+        return b_bar.reshape(ctx.shape), None, None, None, None, None, None, None
 
 
 def solve(matrix: torch.Tensor, rhs: torch.Tensor, keep: Optional[torch.Tensor] = None, rtol: float = 1e-10,
-          max_iterations: Optional[int] = None) -> torch.Tensor:
+          max_iterations: Optional[int] = None, preconditioner: Optional[AmgHierarchy] = None) -> torch.Tensor:
     """`A^-1 rhs` for a symmetric positive definite CSR matrix (rows / columns with keep == 0 masked out), usable inside
-    a loss: gradients flow to `rhs` through a second conjugate-gradient solve."""
+    a loss: gradients flow to `rhs` through a second conjugate-gradient solve.  `preconditioner`: an `amg(matrix, keep)`
+    hierarchy, used by both solves."""
     return _CgSolve.apply(rhs, matrix.crow_indices().to(torch.int32), matrix.col_indices().to(torch.int32), matrix.values(), keep,
-                          rtol, max_iterations)
+                          rtol, max_iterations, preconditioner)
 
 
 class _QuadraticForm(torch.autograd.Function):
     """r^T A^-1 r with ONE solve for value and gradient: d/dr = 2 A^-1 r for symmetric A."""
 
     @staticmethod
-    def forward(ctx, r, crow, col, val, keep, rtol, max_iterations):
-        x, info = cg(crow, col, val, r.detach(), keep, rtol=rtol, max_iterations=max_iterations)
+    def forward(ctx, r, crow, col, val, keep, rtol, max_iterations, preconditioner):
+        x, info = cg(crow, col, val, r.detach(), keep, rtol=rtol, max_iterations=max_iterations, preconditioner=preconditioner)
         if not info.converged:
             raise RuntimeError(f"conjugate gradients stopped at relative residual {info.relative_residual:.3e} after {info.iterations} iterations")
         x = x.reshape(r.shape)
@@ -201,12 +432,13 @@ class _QuadraticForm(torch.autograd.Function):
     @staticmethod
     def backward(ctx, loss_bar):
         (x,) = ctx.saved_tensors
-        return 2.0 * loss_bar * x, None, None, None, None, None, None
+        return 2.0 * loss_bar * x, None, None, None, None, None, None, None
 
 
 def inverse_quadratic_form(matrix: torch.Tensor, residual: torch.Tensor, keep: Optional[torch.Tensor] = None, rtol: float = 1e-10,
-                           max_iterations: Optional[int] = None) -> torch.Tensor:
+                           max_iterations: Optional[int] = None, preconditioner: Optional[AmgHierarchy] = None) -> torch.Tensor:
     """The robust-VPINN loss `r^T G^-1 r` of examples/example_weak.py:84-86,138 on a CSR Gram matrix that cannot be
-    inverted densely: one conjugate-gradient solve gives the value and, since G is symmetric, the gradient 2 G^-1 r."""
+    inverted densely: one conjugate-gradient solve gives the value and, since G is symmetric, the gradient 2 G^-1 r.
+    `preconditioner`: an `amg(matrix, keep)` hierarchy, built once and reused every training step."""
     return _QuadraticForm.apply(residual, matrix.crow_indices().to(torch.int32), matrix.col_indices().to(torch.int32), matrix.values(),
-                                keep, rtol, max_iterations)
+                                keep, rtol, max_iterations, preconditioner)
