@@ -382,6 +382,29 @@ typedef struct tfem_amg_level {
                             int64_t n_cols_c, int64_t n_products, void* workspace,                \
                             int64_t workspace_bytes, int32_t* c_crow, int32_t* c_col, T* c_val,   \
                             int64_t* c_nnz, void* stream);                                         \
+  /* Numeric-only SpGEMM: c_val of C = A B on a known pattern c_crow [n_rows + 1] / c_col (sorted   \
+   * within rows, as tfem_csr_spgemm returns it).  A [n_rows x .] and B CSR.  For the pattern        \
+   * tfem_csr_spgemm returned for the same A and B, c_val equals its c_val bit for bit: each entry   \
+   * is +0 plus its products, each rounded on its own, added in expansion order (A-row entries in   \
+   * stored order, then B-row entries in stored order).  A product whose column C's row lacks is     \
+   * dropped and counted in *n_missing (DEVICE int32, zeroed by the caller; integer atomics only).  \
+   * One warp per row; no workspace, no synchronisation: graph-capturable. */                       \
+  int tfem_csr_spgemm_numeric_##SUF(int64_t n_rows, const int32_t* a_crow, const int32_t* a_col,  \
+                                    const T* a_val, const int32_t* b_crow, const int32_t* b_col,  \
+                                    const T* b_val, const int32_t* c_crow, const int32_t* c_col,  \
+                                    T* c_val, int32_t* n_missing, void* stream);                  \
+  /* AMG refresh, diagonal: diag [n] = a_ii (0 when the row stores none), the diag of             \
+   * tfem_amg_strength without the strength pattern. */                                            \
+  int tfem_amg_diag_##SUF(int64_t n, const int32_t* crow, const int32_t* col, const T* val,        \
+                          T* diag, void* stream);                                                  \
+  /* AMG refresh, smoother operator S = I - omega D^-1 A on A's pattern: wdinv [n] =               \
+   * (1 / diag_i) * omega and s_val [nnz] = delta_ij - wdinv_i * a_ij, each operation rounded on its \
+   * own (the rounding of sparse.amg's torch expressions).  omega must not be NaN. */               \
+  int tfem_amg_smoother_##SUF(int64_t n, const int32_t* crow, const int32_t* col, const T* val,    \
+                              const T* diag, double omega, T* wdinv, T* s_val, void* stream);     \
+  /* Gather with fill: out [n] [k] = src[k] >= 0 ? in[src[k]] : fill (src int32). */                \
+  int tfem_gather_##SUF(int64_t n, const int32_t* src, const T* in, double fill, T* out,           \
+                        void* stream);                                                             \
   /* SURVEY.md 8(f).3 -- fused MLP-at-quadrature-points producer: N(x) and dN/dx of the body of the\
    * reference's FeedForwardNeuralNetwork (model/neural_network.py:50-100: Linear(d,w) act         \
    * {Linear(w,w) act} x n_square Linear(w,1)) by forward-mode differentiation in one pass over    \

@@ -101,6 +101,10 @@ _TYPED = {
     "tfem_amg_vcycle": [POINTER(AmgLevel), c_int32, P, I64, P, P, P],
     "tfem_amg_strength": [I64, P, P, P, c_double, P, P, P],
     "tfem_csr_spgemm": [I64, P, P, P, c_int, P, P, P, I64, I64, I64, P, I64, P, P, P, P, P],
+    "tfem_csr_spgemm_numeric": [I64, P, P, P, P, P, P, P, P, P, P, P],
+    "tfem_amg_diag": [I64, P, P, P, P, P],
+    "tfem_amg_smoother": [I64, P, P, P, P, c_double, P, P, P],
+    "tfem_gather": [I64, P, P, c_double, P, P],
     "tfem_mlp_value_grad": [I64, c_int, c_int, c_int, c_int, P, P, P, P, P],
     "tfem_mlp_value_grad_bwd": [I64, c_int, c_int, c_int, c_int, P, P, P, P, P, c_int, P, P],
     "tfem_iface_pack": [I64, P, P, P, P],

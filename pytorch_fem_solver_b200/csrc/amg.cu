@@ -246,3 +246,96 @@ extern "C" int tfem_amg_aggregate(int64_t n, const int32_t* crow, const int32_t*
   if (cudaMemcpyAsync(n_agg, ids + n, sizeof(int32_t), cudaMemcpyDeviceToDevice, s) != cudaSuccess) return TFEM_ERR_LAUNCH;
   return check_launch();
 }
+
+// ---------------------------------------------------------------------------------------------
+// Numeric refresh of a hierarchy for new values on its pattern (sparse.AmgHierarchy.refresh): the diagonal, the
+// smoother operator S = I - w D^-1 A, and a gather with fill (the finest masked operator from the input values, and
+// R = P^T from P).  Each rounds like the torch expression of sparse.amg it replaces, so a refresh reproduces a build.
+// ---------------------------------------------------------------------------------------------
+namespace tfem {
+
+__device__ __forceinline__ double amg_rcp_rn(double a) { return __drcp_rn(a); }
+__device__ __forceinline__ float amg_rcp_rn(float a) { return __frcp_rn(a); }
+__device__ __forceinline__ double amg_mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float amg_mul_rn(float a, float b) { return __fmul_rn(a, b); }
+
+// wdinv[i] = (1 / a_ii) * omega (torch's `omega / diag` is reciprocal, then product); s[k] = delta_ij - wdinv[i] a_ij
+template <typename T>
+__global__ void __launch_bounds__(256) amg_smoother_kernel(int n, const int32_t* __restrict__ crow, const int32_t* __restrict__ col,
+                                                          const T* __restrict__ val, const T* __restrict__ diag, T omega,
+                                                          T* __restrict__ wdinv, T* __restrict__ s_val) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const T w = amg_mul_rn(amg_rcp_rn(diag[i]), omega);
+  wdinv[i] = w;
+  for (int k = crow[i]; k < crow[i + 1]; ++k) s_val[k] = T(col[k] == i ? 1 : 0) - amg_mul_rn(w, val[k]);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(256) gather_kernel(int n, const int32_t* __restrict__ src, const T* __restrict__ in, T fill,
+                                                    T* __restrict__ out) {
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= n) return;
+  const int s = __ldg(src + k);
+  out[k] = s >= 0 ? __ldg(in + s) : fill;
+}
+
+template <typename T>
+int amg_diag(int64_t n, const int32_t* crow, const int32_t* col, const T* val, T* diag, void* stream) {
+  if (n < 0) return TFEM_ERR_BAD_ARG;
+  if (n == 0) return TFEM_OK;
+  if (!crow || !col || !val || !diag) return TFEM_ERR_BAD_ARG;
+  if (n >= kMaxIndex) return TFEM_ERR_TOO_LARGE;
+  amg_diag_kernel<T><<<blocks_for(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>((int)n, crow, col, val, diag);
+  return check_launch();
+}
+
+template <typename T>
+int amg_smoother(int64_t n, const int32_t* crow, const int32_t* col, const T* val, const T* diag, double omega, T* wdinv, T* s_val,
+                 void* stream) {
+  if (n < 0 || !(omega == omega)) return TFEM_ERR_BAD_ARG;
+  if (n == 0) return TFEM_OK;
+  if (!crow || !col || !val || !diag || !wdinv || !s_val) return TFEM_ERR_BAD_ARG;
+  if (n >= kMaxIndex) return TFEM_ERR_TOO_LARGE;
+  amg_smoother_kernel<T><<<blocks_for(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>((int)n, crow, col, val, diag, T(omega),
+                                                                                              wdinv, s_val);
+  return check_launch();
+}
+
+template <typename T>
+int gather(int64_t n, const int32_t* src, const T* in, double fill, T* out, void* stream) {
+  if (n < 0) return TFEM_ERR_BAD_ARG;
+  if (n == 0) return TFEM_OK;
+  if (!src || !in || !out) return TFEM_ERR_BAD_ARG;
+  if (n >= kMaxIndex) return TFEM_ERR_TOO_LARGE;
+  gather_kernel<T><<<blocks_for(n, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>((int)n, src, in, T(fill), out);
+  return check_launch();
+}
+
+}  // namespace tfem
+
+extern "C" int tfem_amg_diag_f64(int64_t n, const int32_t* crow, const int32_t* col, const double* val, double* diag, void* stream) {
+  return tfem::amg_diag<double>(n, crow, col, val, diag, stream);
+}
+
+extern "C" int tfem_amg_diag_f32(int64_t n, const int32_t* crow, const int32_t* col, const float* val, float* diag, void* stream) {
+  return tfem::amg_diag<float>(n, crow, col, val, diag, stream);
+}
+
+extern "C" int tfem_amg_smoother_f64(int64_t n, const int32_t* crow, const int32_t* col, const double* val, const double* diag,
+                                     double omega, double* wdinv, double* s_val, void* stream) {
+  return tfem::amg_smoother<double>(n, crow, col, val, diag, omega, wdinv, s_val, stream);
+}
+
+extern "C" int tfem_amg_smoother_f32(int64_t n, const int32_t* crow, const int32_t* col, const float* val, const float* diag,
+                                     double omega, float* wdinv, float* s_val, void* stream) {
+  return tfem::amg_smoother<float>(n, crow, col, val, diag, omega, wdinv, s_val, stream);
+}
+
+extern "C" int tfem_gather_f64(int64_t n, const int32_t* src, const double* in, double fill, double* out, void* stream) {
+  return tfem::gather<double>(n, src, in, fill, out, stream);
+}
+
+extern "C" int tfem_gather_f32(int64_t n, const int32_t* src, const float* in, double fill, float* out, void* stream) {
+  return tfem::gather<float>(n, src, in, fill, out, stream);
+}

@@ -344,3 +344,105 @@ extern "C" int tfem_csr_spgemm_f32(int64_t n_rows_a, const int32_t* a_crow, cons
   return tfem::csr_spgemm<float>(n_rows_a, a_crow, a_col, a_val, transpose, b_crow, b_col, b_val, n_rows_c, n_cols_c, n_products, workspace,
                                  workspace_bytes, c_crow, c_col, c_val, c_nnz, stream);
 }
+
+// ---------------------------------------------------------------------------------------------
+// Numeric-only SpGEMM: the values of C = A B on a known pattern (c_crow, c_col sorted within rows, as
+// tfem_csr_spgemm returns it), for a refresh of the AMG hierarchy with new values (sparse.AmgHierarchy.refresh).
+// Bitwise equal to tfem_csr_spgemm's c_val: each entry is +0 plus its products added left to right in expansion
+// order (A-row entries in stored order, then B-row entries in stored order) -- the order the stable sort gives the
+// segmented sum -- and each product is rounded on its own (__dmul_rn / __fmul_rn: no contraction into an FMA).
+// One warp per C row.  The warp takes the products of one A entry 32 at a time; each lane forms one product and finds
+// its C slot by binary search; then every lane walks the staged products in order and adds those of the slots it
+// owns (slot = lane + 32 t) to registers.  Rows longer than 32 * kNumericSlots run in several passes over the same
+// products.  No sort, no workspace, no float atomics; products whose column C's row lacks are dropped and counted.
+// ---------------------------------------------------------------------------------------------
+namespace tfem {
+
+constexpr int kNumericSlots = 4;  // C slots per lane and pass: rows up to 128 entries in one pass
+
+__device__ __forceinline__ double mul_rn(double a, double b) { return __dmul_rn(a, b); }
+__device__ __forceinline__ float mul_rn(float a, float b) { return __fmul_rn(a, b); }
+
+template <typename T>
+__global__ void __launch_bounds__(256) spgemm_numeric_kernel(int n_rows, const int32_t* __restrict__ a_crow, const int32_t* __restrict__ a_col,
+                                                             const T* __restrict__ a_val, const int32_t* __restrict__ b_crow,
+                                                             const int32_t* __restrict__ b_col, const T* __restrict__ b_val,
+                                                             const int32_t* __restrict__ c_crow, const int32_t* __restrict__ c_col,
+                                                             T* __restrict__ c_val, int32_t* __restrict__ n_missing) {
+  const int row = (int)(((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+  const int lane = threadIdx.x & 31;
+  if (row >= n_rows) return;  // warp-uniform
+  const int c_begin = __ldg(c_crow + row), c_len = __ldg(c_crow + row + 1) - c_begin;
+  const int a_begin = __ldg(a_crow + row), a_end = __ldg(a_crow + row + 1);
+  const int32_t* cc = c_col + c_begin;
+  int missing = 0;
+  for (int chunk = 0; chunk == 0 || chunk < c_len; chunk += 32 * kNumericSlots) {
+    T acc[kNumericSlots];
+#pragma unroll
+    for (int t = 0; t < kNumericSlots; ++t) acc[t] = T(0);
+    for (int k = a_begin; k < a_end; ++k) {
+      const int j = __ldg(a_col + k);
+      const T a = __ldg(a_val + k);
+      const int b_begin = __ldg(b_crow + j), b_end = __ldg(b_crow + j + 1);
+      for (int base = b_begin; base < b_end; base += 32) {
+        const int q = base + lane;
+        int slot = -1;
+        T prod = T(0);
+        if (q < b_end) {
+          prod = mul_rn(a, __ldg(b_val + q));
+          const int c = __ldg(b_col + q);
+          int lo = 0, hi = c_len;
+          while (lo < hi) {
+            const int mid = (lo + hi) >> 1;
+            if (__ldg(cc + mid) < c) lo = mid + 1;
+            else hi = mid;
+          }
+          if (lo < c_len && __ldg(cc + lo) == c) slot = lo - chunk;
+          else if (chunk == 0) ++missing;
+        }
+        const int staged = min(32, b_end - base);
+        for (int s = 0; s < staged; ++s) {
+          const int sl = __shfl_sync(0xffffffffu, slot, s);
+          const T p = __shfl_sync(0xffffffffu, prod, s);
+#pragma unroll
+          for (int t = 0; t < kNumericSlots; ++t)
+            if (sl == lane + 32 * t) acc[t] += p;
+        }
+      }
+    }
+#pragma unroll
+    for (int t = 0; t < kNumericSlots; ++t) {
+      const int sl = chunk + lane + 32 * t;
+      if (sl < c_len) c_val[c_begin + sl] = acc[t];
+    }
+  }
+  missing = __reduce_add_sync(0xffffffffu, missing);
+  if (lane == 0 && missing) atomicAdd(n_missing, missing);  // integer count: order does not matter
+}
+
+template <typename T>
+int csr_spgemm_numeric(int64_t n_rows, const int32_t* a_crow, const int32_t* a_col, const T* a_val, const int32_t* b_crow,
+                       const int32_t* b_col, const T* b_val, const int32_t* c_crow, const int32_t* c_col, T* c_val, int32_t* n_missing,
+                       void* stream) {
+  if (n_rows < 0) return TFEM_ERR_BAD_ARG;
+  if (n_rows == 0) return TFEM_OK;
+  if (!a_crow || !a_col || !a_val || !b_crow || !b_col || !b_val || !c_crow || !c_col || !c_val || !n_missing) return TFEM_ERR_BAD_ARG;
+  if (n_rows > kMaxIndex / 32) return TFEM_ERR_TOO_LARGE;
+  spgemm_numeric_kernel<T><<<blocks_for(n_rows * 32, 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+      (int)n_rows, a_crow, a_col, a_val, b_crow, b_col, b_val, c_crow, c_col, c_val, n_missing);
+  return check_launch();
+}
+
+}  // namespace tfem
+
+extern "C" int tfem_csr_spgemm_numeric_f64(int64_t n_rows, const int32_t* a_crow, const int32_t* a_col, const double* a_val,
+                                           const int32_t* b_crow, const int32_t* b_col, const double* b_val, const int32_t* c_crow,
+                                           const int32_t* c_col, double* c_val, int32_t* n_missing, void* stream) {
+  return tfem::csr_spgemm_numeric<double>(n_rows, a_crow, a_col, a_val, b_crow, b_col, b_val, c_crow, c_col, c_val, n_missing, stream);
+}
+
+extern "C" int tfem_csr_spgemm_numeric_f32(int64_t n_rows, const int32_t* a_crow, const int32_t* a_col, const float* a_val,
+                                           const int32_t* b_crow, const int32_t* b_col, const float* b_val, const int32_t* c_crow,
+                                           const int32_t* c_col, float* c_val, int32_t* n_missing, void* stream) {
+  return tfem::csr_spgemm_numeric<float>(n_rows, a_crow, a_col, a_val, b_crow, b_col, b_val, c_crow, c_col, c_val, n_missing, stream);
+}

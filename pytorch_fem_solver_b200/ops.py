@@ -336,6 +336,49 @@ def csr_spgemm(a: Tuple[Tensor, Tensor, Tensor], n_cols_a: int, b: Optional[Tupl
     return c_crow, c_col[:nnz].clone(), c_val[:nnz].clone()
 
 
+def csr_spgemm_numeric(a: Tuple[Tensor, Tensor, Tensor], b: Tuple[Tensor, Tensor, Tensor], c_crow: Tensor, c_col: Tensor,
+                       out: Optional[Tensor] = None, n_missing: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
+    """(c_val, n_missing): the values of C = A B on the pattern (c_crow, c_col), bitwise those `csr_spgemm` gives on its
+    own pattern (tfem_csr_spgemm_numeric).  `out` receives c_val in place; products outside the pattern are dropped and
+    counted into the int32 device counter `n_missing` (a new zeroed one when None)."""
+    a_crow, a_col, a_val = a
+    b_crow, b_col, b_val = b
+    device = check_cuda(a_crow, a_col, a_val, b_crow, b_col, b_val, c_crow, c_col, out, n_missing)
+    if out is None:
+        out = torch.empty(c_col.shape[0], dtype=a_val.dtype, device=device)
+    if n_missing is None:
+        n_missing = torch.zeros(1, dtype=torch.int32, device=device)
+    # an empty A, B or C has no storage; the kernel reads nothing of it but the entry point wants a pointer
+    a_col, a_val, b_col, b_val, c_col, c_val = (t if t.numel() else t.new_empty(1) for t in (a_col, a_val, b_col, b_val, c_col, out))
+    call("tfem_csr_spgemm_numeric", a_val.dtype, device, a_crow.shape[0] - 1, ptr(a_crow), ptr(a_col), ptr(a_val), ptr(b_crow), ptr(b_col),
+         ptr(b_val), ptr(c_crow), ptr(c_col), ptr(c_val), ptr(n_missing))
+    return out, n_missing
+
+
+def amg_diag(crow: Tensor, col: Tensor, val: Tensor) -> Tensor:
+    """diag [n] of a CSR matrix (0 where a row stores none): the diagonal `amg_strength` returns."""
+    device = check_cuda(crow, col, val)
+    diag = torch.empty(crow.shape[0] - 1, dtype=val.dtype, device=device)
+    call("tfem_amg_diag", val.dtype, device, crow.shape[0] - 1, ptr(crow), ptr(col), ptr(val), ptr(diag))
+    return diag
+
+
+def amg_smoother(crow: Tensor, col: Tensor, val: Tensor, diag: Tensor, omega: float, wdinv: Tensor, s_val: Tensor) -> None:
+    """wdinv = omega / diag and s_val = I - wdinv A on A's pattern, in place, rounded as `sparse.amg`'s torch expressions."""
+    device = check_cuda(crow, col, val, diag, wdinv, s_val)
+    call("tfem_amg_smoother", val.dtype, device, crow.shape[0] - 1, ptr(crow), ptr(col), ptr(val), ptr(diag), float(omega), ptr(wdinv),
+         ptr(s_val))
+
+
+def gather_fill(src: Tensor, values: Tensor, fill: float, out: Tensor) -> Tensor:
+    """out[k] = values[src[k]] where src[k] >= 0, else fill (src int32), in place (tfem_gather)."""
+    device = check_cuda(src, values, out)
+    if out.shape[0] != src.shape[0] or out.dtype != values.dtype:
+        raise TfemError("gather_fill: out must have src's length and the values' dtype")
+    call("tfem_gather", values.dtype, device, src.shape[0], ptr(src), ptr(values), float(fill), ptr(out))
+    return out
+
+
 def amg_levels_struct(hierarchy):
     """ctypes array of struct tfem_amg_level over the device tensors of an `sparse.AmgHierarchy` (kept alive by it)."""
     levels = hierarchy.levels

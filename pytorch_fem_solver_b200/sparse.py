@@ -11,6 +11,8 @@ the device; the host looks at the residual only every `check_every` iterations.
 `amg()` builds a smoothed-aggregation algebraic multigrid hierarchy once, on the device, and
 `preconditioner=` replaces Jacobi by one V-cycle of it per iteration (`tfem_pcg_iteration`); the
 Gram matrix of a training loop is fixed, so one hierarchy serves every step (DESIGN.md §8(f).1).
+`amg(..., refreshable=True)` also keeps the symbolic data for `AmgHierarchy.refresh`, which recomputes
+every value for a new matrix on the same pattern without re-aggregating (moving meshes, K + beta M).
 """
 
 from __future__ import annotations
@@ -219,6 +221,41 @@ class AmgLevel:
 
 
 @dataclass
+class AmgLevelPattern:
+    """What a refresh of one level needs beyond the level itself: the tentative prolongator T (its values depend only on
+    the aggregates), the pattern and values of the intermediate A P, and r_map (R entry k is P entry r_map[k])."""
+
+    t_crow: torch.Tensor
+    t_col: torch.Tensor
+    t_val: torch.Tensor
+    ap_crow: torch.Tensor
+    ap_col: torch.Tensor
+    ap_val: torch.Tensor
+    r_map: torch.Tensor
+
+
+@dataclass
+class AmgPattern:
+    """The symbolic data of a refreshable hierarchy: the input pattern it was built for, the gather map src from input
+    values to the finest operator (M A M) + (I - M) (-1: a masked diagonal, set to 1), each level's AmgLevelPattern and
+    the coarsest operator as CSR."""
+
+    crow: torch.Tensor
+    col: torch.Tensor
+    src: torch.Tensor
+    levels: List[AmgLevelPattern]
+    coarse_crow: torch.Tensor
+    coarse_col: torch.Tensor
+    coarse_val: torch.Tensor
+
+    def tensors(self) -> List[torch.Tensor]:
+        out = [self.crow, self.col, self.src, self.coarse_crow, self.coarse_col, self.coarse_val]
+        for lev in self.levels:
+            out += [lev.t_crow, lev.t_col, lev.t_val, lev.ap_crow, lev.ap_col, lev.ap_val, lev.r_map]
+        return out
+
+
+@dataclass
 class AmgHierarchy:
     """The hierarchy `amg()` builds for one matrix and keep mask; pass it as `preconditioner=`.
 
@@ -231,6 +268,7 @@ class AmgHierarchy:
     nnz: int
     theta: float
     _struct: object = field(default=None, repr=False)
+    pattern: Optional[AmgPattern] = field(default=None, repr=False)  # amg(..., refreshable=True) only
 
     @property
     def n(self) -> int:
@@ -285,6 +323,59 @@ class AmgHierarchy:
         if not torch.equal(keep, self.keep):
             raise ValueError("the AMG hierarchy was built for another keep mask")
 
+    def refresh(self, matrix: torch.Tensor) -> "AmgHierarchy":
+        """Recompute every value of this hierarchy for new matrix values on the pattern it was built from; returns self.
+
+        `matrix`: a sparse CSR tensor with the built pattern, or a 1-D array of values aligned with it (like
+        `layout="values"`).  The aggregates, the keep mask and every sparsity pattern stay; per level the operator, its
+        diagonal, rho (the same power iteration as the build), omega, omega D^-1, P = (I - omega D^-1 A) T, R = P^T, A P
+        and A_c are recomputed, then the dense coarsest inverse.  Every device tensor keeps its storage, so the
+        hierarchy stays valid wherever it is already passed as `preconditioner=`.  A refresh with the matrix of the
+        build reproduces the build bit for bit.
+
+        It does not re-aggregate: when the strength pattern of the new matrix differs completely (e.g. another
+        anisotropy), build a new hierarchy instead.  A hierarchy refreshed between the forward and the backward of
+        `solve` preconditions the adjoint solve with the new values; that solve still converges to the adjoint of the
+        saved matrix, which it multiplies by.
+
+        ValueError, with nothing modified, for a hierarchy built without `refreshable=True`, a matrix of another size,
+        nnz, dtype, device or pattern, or a value array of the wrong length."""
+        pat = self.pattern
+        if pat is None:
+            raise ValueError("the AMG hierarchy was not built with refreshable=True")
+        if isinstance(matrix, torch.Tensor) and matrix.layout == torch.sparse_csr:
+            crow, col, val = matrix.crow_indices(), matrix.col_indices(), matrix.values()
+            self.check(crow, val, self.keep)
+            if not (torch.equal(crow.to(torch.int32), pat.crow) and torch.equal(col.to(torch.int32), pat.col)):
+                raise ValueError("the matrix has another sparsity pattern than the AMG hierarchy was built for")
+        else:
+            val = matrix
+            if val.dim() != 1 or val.shape[0] != self.nnz or val.dtype != self.dtype or val.device != self.device:
+                raise ValueError(f"a value array of the AMG hierarchy is a 1-D {self.dtype} tensor of {self.nnz} entries on {self.device}, "
+                                 f"not a {val.dim()}-D {val.dtype} tensor of shape {tuple(val.shape)} on {val.device}")
+        val = val.contiguous()
+        missing = torch.zeros(1, dtype=torch.int32, device=self.device)
+        ops.gather_fill(pat.src, val, 1.0, self.levels[0].a_val if self.levels else pat.coarse_val)
+        for level, (lev, lp) in enumerate(zip(self.levels, pat.levels)):
+            a = (lev.a_crow, lev.a_col, lev.a_val)
+            diag = ops.amg_diag(*a)
+            rho = _spectral_radius(*a, 1.0 / diag, level)
+            omega = 4.0 / (3.0 * rho)
+            s_val = torch.empty_like(lev.a_val)
+            ops.amg_smoother(*a, diag, omega, lev.wdinv, s_val)
+            p = (lev.p_crow, lev.p_col, lev.p_val)
+            ops.csr_spgemm_numeric((lev.a_crow, lev.a_col, s_val), (lp.t_crow, lp.t_col, lp.t_val), lev.p_crow, lev.p_col, lev.p_val, missing)
+            ops.gather_fill(lp.r_map, lev.p_val, 0.0, lev.r_val)
+            ops.csr_spgemm_numeric(a, p, lp.ap_crow, lp.ap_col, lp.ap_val, missing)
+            nxt = self.levels[level + 1] if level + 1 < len(self.levels) else None
+            c = (nxt.a_crow, nxt.a_col, nxt.a_val) if nxt is not None else (pat.coarse_crow, pat.coarse_col, pat.coarse_val)
+            ops.csr_spgemm_numeric((lev.r_crow, lev.r_col, lev.r_val), (lp.ap_crow, lp.ap_col, lp.ap_val), c[0], c[1], c[2], missing)
+            lev.rho, lev.omega = rho, omega
+        self.coarse_inv.copy_(_dense_inverse(pat.coarse_crow, pat.coarse_col, pat.coarse_val))
+        if int(missing.item()) != 0:  # the patterns are those of the build: a product outside them is an internal error
+            raise RuntimeError(f"AMG refresh: {int(missing.item())} products fell outside the hierarchy's patterns")
+        return self
+
 
 def _hash32(i: torch.Tensor, salt: int) -> torch.Tensor:
     """oracle/amg_oracle.py hash32 in int64 arithmetic (products wrap; the low 32 bits are exact)."""
@@ -312,6 +403,36 @@ def _masked_operator(crow, col, val, keep8):
     return new_crow, col[live].contiguous(), v[live].contiguous()
 
 
+def _masked_operator_map(crow, col, keep8):
+    """src [nnz of the masked operator]: the input entry each entry of `_masked_operator` takes (-1: a masked
+    diagonal, which is 1)."""
+    index = torch.arange(col.shape[0], dtype=torch.int32, device=col.device)
+    if keep8 is None:
+        return index
+    n = crow.shape[0] - 1
+    row = torch.repeat_interleave(torch.arange(n, device=col.device), (crow[1:] - crow[:-1]).long())
+    k = keep8 != 0
+    on_diag = row == col.long()
+    live = (k[row] & k[col.long()]) | on_diag
+    src = torch.where(on_diag & ~k[row], torch.full_like(index, -1), index)
+    return src[live].contiguous()
+
+
+def _transpose_map(p_crow, p_col):
+    """r_map: R = P^T entry k is P entry r_map[k] (a stable sort of P's (column, row) keys, R's CSR order)."""
+    n = p_crow.shape[0] - 1
+    row = torch.repeat_interleave(torch.arange(n, device=p_col.device), (p_crow[1:] - p_crow[:-1]).long())
+    key = p_col.long() * n + row
+    return torch.argsort(key, stable=True).to(torch.int32)
+
+
+def _dense_inverse(a_crow, a_col, a_val):
+    n_c = a_crow.shape[0] - 1
+    dense = torch.zeros((n_c, n_c), dtype=a_val.dtype, device=a_val.device)
+    dense[torch.repeat_interleave(torch.arange(n_c, device=a_val.device), (a_crow[1:] - a_crow[:-1]).long()), a_col.long()] = a_val
+    return torch.linalg.inv(dense).contiguous()
+
+
 def _spectral_radius(crow, col, val, inv_diag, level: int) -> float:
     """rho(D^-1 A) by power iteration from a hash-generated (reproducible) start vector."""
     n = crow.shape[0] - 1
@@ -326,7 +447,7 @@ def _spectral_radius(crow, col, val, inv_diag, level: int) -> float:
 
 
 def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float = 0.08, max_coarse: int = 1000,
-        max_levels: int = 12) -> AmgHierarchy:
+        max_levels: int = 12, refreshable: bool = False) -> AmgHierarchy:
     """Smoothed-aggregation AMG hierarchy of the operator `cg` solves, (M A M) + (I - M), M = diag(keep), for a
     symmetric positive definite CSR `matrix`; one-time set-up on the device.
 
@@ -334,7 +455,11 @@ def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float 
     T = 1 / sqrt(|aggregate|) (nodes without strong connections stay unaggregated: the smoother alone handles them);
     rho(D^-1 A) by 15 power iterations; P = (I - omega D^-1 A) T, omega = 4 / (3 rho); R = P^T; A_c = R A P by the
     deterministic SpGEMM.  Coarsening stops at <= max_coarse rows or max_levels levels; the coarsest operator is
-    inverted densely.  The result is reproducible run to run."""
+    inverted densely.  The result is reproducible run to run.
+
+    `refreshable=True` also keeps what `AmgHierarchy.refresh` needs to recompute the values for a new matrix on the same
+    pattern (the finest gather map, T, the pattern of A P and the R-from-P map per level, the coarsest pattern); the
+    hierarchy itself is the same bit for bit."""
     crow, col, val = matrix.crow_indices().to(torch.int32), matrix.col_indices().to(torch.int32), matrix.values()
     n = crow.shape[0] - 1
     keep8 = None if keep is None else keep.reshape(-1).to(device=val.device, dtype=torch.uint8).contiguous()
@@ -342,6 +467,7 @@ def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float 
         raise ValueError("keep mask length does not match the matrix")
     a = _masked_operator(crow, col, val, keep8)
     levels: List[AmgLevel] = []
+    patterns: List[AmgLevelPattern] = []
     while a[0].shape[0] - 1 > max_coarse and len(levels) + 1 < max_levels:
         level = len(levels)
         a_crow, a_col, a_val = a
@@ -366,17 +492,27 @@ def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float 
         ap = ops.csr_spgemm(a, n_l, p, n_agg)
         a_c = ops.csr_spgemm(r, n_l, ap, n_agg)
         levels.append(AmgLevel(n_l, n_agg, a_crow, a_col, a_val, *p, *r, wdinv, agg, rho, omega))
+        if refreshable:
+            r_map = _transpose_map(p[0], p[1])
+            if not torch.equal(p[2][r_map.long()].view(_bits(p[2].dtype)), r[2].view(_bits(r[2].dtype))):
+                raise RuntimeError("AMG set-up: R is not P^T gathered through the transpose map")
+            patterns.append(AmgLevelPattern(t_crow, t_col, t_val, ap[0], ap[1], ap[2], r_map))
         a = a_c
     a_crow, a_col, a_val = a
     n_c = a_crow.shape[0] - 1
     if n_c > MAX_DENSE_COARSE:
         raise ValueError(f"coarsening stopped at {n_c} rows, more than the dense coarsest solve takes ({MAX_DENSE_COARSE}); "
                          "raise max_levels or lower theta")
-    dense = torch.zeros((n_c, n_c), dtype=a_val.dtype, device=a_val.device)
-    dense[torch.repeat_interleave(torch.arange(n_c, device=a_val.device), (a_crow[1:] - a_crow[:-1]).long()), a_col.long()] = a_val
-    coarse_inv = torch.linalg.inv(dense).contiguous()
+    coarse_inv = _dense_inverse(a_crow, a_col, a_val)
     keep_all = torch.ones(n, dtype=torch.uint8, device=val.device) if keep8 is None else keep8.clone()
-    return AmgHierarchy(levels, coarse_inv, a_col.shape[0], keep_all, val.shape[0], theta)
+    pattern = None
+    if refreshable:
+        pattern = AmgPattern(crow, col, _masked_operator_map(crow, col, keep8), patterns, a_crow, a_col, a_val)
+    return AmgHierarchy(levels, coarse_inv, a_col.shape[0], keep_all, val.shape[0], theta, pattern=pattern)
+
+
+def _bits(dtype: torch.dtype) -> torch.dtype:
+    return torch.int64 if dtype == torch.float64 else torch.int32
 
 
 class _CgSolve(torch.autograd.Function):
