@@ -248,9 +248,9 @@ extern "C" int tfem_amg_aggregate(int64_t n, const int32_t* crow, const int32_t*
 }
 
 // ---------------------------------------------------------------------------------------------
-// Numeric refresh of a hierarchy for new values on its pattern (sparse.AmgHierarchy.refresh): the diagonal, the
-// smoother operator S = I - w D^-1 A, and a gather with fill (the finest masked operator from the input values, and
-// R = P^T from P).  Each rounds like the torch expression of sparse.amg it replaces, so a refresh reproduces a build.
+// Per-level values shared by the set-up (sparse.amg) and the numeric refresh (sparse.AmgHierarchy.refresh): the
+// diagonal, the smoother operator S = I - w D^-1 A, and a gather with fill (the finest masked operator from the input
+// values, and R = P^T from P).
 // ---------------------------------------------------------------------------------------------
 namespace tfem {
 

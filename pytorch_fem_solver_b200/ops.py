@@ -309,29 +309,21 @@ def amg_aggregate(crow: Tensor, col: Tensor, strong: Tensor, level: int) -> Tupl
     return agg, int(counter.item())
 
 
-def csr_spgemm(a: Tuple[Tensor, Tensor, Tensor], n_cols_a: int, b: Optional[Tuple[Tensor, Tensor, Tensor]] = None,
-               n_cols_b: int = 0, transpose: bool = False) -> Tuple[Tensor, Tensor, Tensor]:
-    """C = op(A) B as CSR (crow, col, val), op(A) = A^T with `transpose`, B = identity when None (tfem_csr_spgemm)."""
+def csr_spgemm(a: Tuple[Tensor, Tensor, Tensor], n_cols_a: int, b: Tuple[Tensor, Tensor, Tensor], n_cols_b: int) -> Tuple[Tensor, Tensor, Tensor]:
+    """C = A B as CSR (crow, col, val) for A with n_cols_a columns and B with n_cols_b (tfem_csr_spgemm; the device
+    product reads A's column count from B's row pointer)."""
     a_crow, a_col, a_val = a
-    device = check_cuda(a_crow, a_col, a_val, *(b or ()))
-    n_rows_a = a_crow.shape[0] - 1
-    n_rows_c = n_cols_a if transpose else n_rows_a
-    n_cols_c = (n_rows_a if transpose else n_cols_a) if b is None else n_cols_b
-    a_len = (a_crow[1:] - a_crow[:-1]).long()
-    if b is None:
-        n_products = a_col.shape[0]
-    else:
-        b_len = (b[0][1:] - b[0][:-1]).long()
-        n_products = int((a_len * b_len).sum()) if transpose else int(b_len[a_col.long()].sum())
-    workspace = torch.empty(_workspace("tfem_csr_spgemm_workspace", n_rows_a, n_products), dtype=torch.uint8, device=device)
-    c_crow = torch.empty(n_rows_c + 1, dtype=torch.int32, device=device)
+    b_crow, b_col, b_val = b
+    device = check_cuda(a_crow, a_col, a_val, b_crow, b_col, b_val)
+    n_rows = a_crow.shape[0] - 1
+    n_products = int((b_crow[1:] - b_crow[:-1]).long()[a_col.long()].sum())
+    workspace = torch.empty(_workspace("tfem_csr_spgemm_workspace", n_rows, n_products), dtype=torch.uint8, device=device)
+    c_crow = torch.empty(n_rows + 1, dtype=torch.int32, device=device)
     c_col = torch.empty(max(n_products, 1), dtype=torch.int32, device=device)
     c_val = torch.empty(max(n_products, 1), dtype=a_val.dtype, device=device)
     c_nnz = torch.zeros(1, dtype=torch.int64, device=device)
-    b_crow, b_col, b_val = b if b is not None else (None, None, None)
-    call("tfem_csr_spgemm", a_val.dtype, device, n_rows_a, ptr(a_crow), ptr(a_col), ptr(a_val), int(transpose), ptr(b_crow), ptr(b_col),
-         ptr(b_val), n_rows_c, max(n_cols_c, 1), n_products, ptr(workspace), workspace.numel(), ptr(c_crow), ptr(c_col), ptr(c_val),
-         ptr(c_nnz))
+    call("tfem_csr_spgemm", a_val.dtype, device, n_rows, ptr(a_crow), ptr(a_col), ptr(a_val), 0, ptr(b_crow), ptr(b_col), ptr(b_val),
+         n_rows, max(n_cols_b, 1), n_products, ptr(workspace), workspace.numel(), ptr(c_crow), ptr(c_col), ptr(c_val), ptr(c_nnz))
     nnz = int(c_nnz.item())
     return c_crow, c_col[:nnz].clone(), c_val[:nnz].clone()
 
@@ -364,7 +356,7 @@ def amg_diag(crow: Tensor, col: Tensor, val: Tensor) -> Tensor:
 
 
 def amg_smoother(crow: Tensor, col: Tensor, val: Tensor, diag: Tensor, omega: float, wdinv: Tensor, s_val: Tensor) -> None:
-    """wdinv = omega / diag and s_val = I - wdinv A on A's pattern, in place, rounded as `sparse.amg`'s torch expressions."""
+    """wdinv = omega / diag and s_val = I - wdinv A on A's pattern, in place, rounded as torch rounds those expressions."""
     device = check_cuda(crow, col, val, diag, wdinv, s_val)
     call("tfem_amg_smoother", val.dtype, device, crow.shape[0] - 1, ptr(crow), ptr(col), ptr(val), ptr(diag), float(omega), ptr(wdinv),
          ptr(s_val))

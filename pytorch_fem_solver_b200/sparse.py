@@ -353,24 +353,15 @@ class AmgHierarchy:
             if val.dim() != 1 or val.shape[0] != self.nnz or val.dtype != self.dtype or val.device != self.device:
                 raise ValueError(f"a value array of the AMG hierarchy is a 1-D {self.dtype} tensor of {self.nnz} entries on {self.device}, "
                                  f"not a {val.dim()}-D {val.dtype} tensor of shape {tuple(val.shape)} on {val.device}")
-        val = val.contiguous()
         missing = torch.zeros(1, dtype=torch.int32, device=self.device)
-        ops.gather_fill(pat.src, val, 1.0, self.levels[0].a_val if self.levels else pat.coarse_val)
+        ops.gather_fill(pat.src, val.contiguous(), 1.0, self.levels[0].a_val if self.levels else pat.coarse_val)
         for level, (lev, lp) in enumerate(zip(self.levels, pat.levels)):
             a = (lev.a_crow, lev.a_col, lev.a_val)
-            diag = ops.amg_diag(*a)
-            rho = _spectral_radius(*a, 1.0 / diag, level)
-            omega = 4.0 / (3.0 * rho)
-            s_val = torch.empty_like(lev.a_val)
-            ops.amg_smoother(*a, diag, omega, lev.wdinv, s_val)
-            p = (lev.p_crow, lev.p_col, lev.p_val)
-            ops.csr_spgemm_numeric((lev.a_crow, lev.a_col, s_val), (lp.t_crow, lp.t_col, lp.t_val), lev.p_crow, lev.p_col, lev.p_val, missing)
-            ops.gather_fill(lp.r_map, lev.p_val, 0.0, lev.r_val)
-            ops.csr_spgemm_numeric(a, p, lp.ap_crow, lp.ap_col, lp.ap_val, missing)
             nxt = self.levels[level + 1] if level + 1 < len(self.levels) else None
             c = (nxt.a_crow, nxt.a_col, nxt.a_val) if nxt is not None else (pat.coarse_crow, pat.coarse_col, pat.coarse_val)
-            ops.csr_spgemm_numeric((lev.r_crow, lev.r_col, lev.r_val), (lp.ap_crow, lp.ap_col, lp.ap_val), c[0], c[1], c[2], missing)
-            lev.rho, lev.omega = rho, omega
+            out = ((lev.p_crow, lev.p_col, lev.p_val), ((lev.r_crow, lev.r_col, lev.r_val), lp.r_map), (lp.ap_crow, lp.ap_col, lp.ap_val), c)
+            lev.rho, lev.omega, *_ = _level_values(a, ops.amg_diag(*a), (lp.t_crow, lp.t_col, lp.t_val), level, lev.n_coarse, lev.wdinv,
+                                                   out, missing)
         self.coarse_inv.copy_(_dense_inverse(pat.coarse_crow, pat.coarse_col, pat.coarse_val))
         if int(missing.item()) != 0:  # the patterns are those of the build: a product outside them is an internal error
             raise RuntimeError(f"AMG refresh: {int(missing.item())} products fell outside the hierarchy's patterns")
@@ -388,42 +379,65 @@ def _hash32(i: torch.Tensor, salt: int) -> torch.Tensor:
     return h ^ (h >> 16)
 
 
-def _masked_operator(crow, col, val, keep8):
-    """(M A M) + (I - M): masked rows and columns dropped, their diagonals set to 1."""
-    if keep8 is None:
-        return crow, col, val.clone()
-    n = crow.shape[0] - 1
-    row = torch.repeat_interleave(torch.arange(n, device=col.device), (crow[1:] - crow[:-1]).long())
-    k = keep8 != 0
-    on_diag = row == col.long()
-    live = (k[row] & k[col.long()]) | on_diag
-    v = torch.where(on_diag & ~k[row], torch.ones_like(val), val)
-    counts = torch.bincount(row[live], minlength=n)
-    new_crow = torch.cat([counts.new_zeros(1), torch.cumsum(counts, 0)]).to(torch.int32)
-    return new_crow, col[live].contiguous(), v[live].contiguous()
-
-
 def _masked_operator_map(crow, col, keep8):
-    """src [nnz of the masked operator]: the input entry each entry of `_masked_operator` takes (-1: a masked
-    diagonal, which is 1)."""
+    """(crow, col, src) of (M A M) + (I - M): masked rows and columns dropped, their diagonals kept.  Entry k takes
+    input entry src[k], or is 1 where src[k] = -1 (a masked diagonal); `ops.gather_fill(src, val, 1.0, out)` fills it."""
     index = torch.arange(col.shape[0], dtype=torch.int32, device=col.device)
     if keep8 is None:
-        return index
+        return crow, col, index
     n = crow.shape[0] - 1
     row = torch.repeat_interleave(torch.arange(n, device=col.device), (crow[1:] - crow[:-1]).long())
     k = keep8 != 0
     on_diag = row == col.long()
     live = (k[row] & k[col.long()]) | on_diag
     src = torch.where(on_diag & ~k[row], torch.full_like(index, -1), index)
-    return src[live].contiguous()
+    counts = torch.bincount(row[live], minlength=n)
+    new_crow = torch.cat([counts.new_zeros(1), torch.cumsum(counts, 0)]).to(torch.int32)
+    return new_crow, col[live].contiguous(), src[live].contiguous()
 
 
-def _transpose_map(p_crow, p_col):
-    """r_map: R = P^T entry k is P entry r_map[k] (a stable sort of P's (column, row) keys, R's CSR order)."""
-    n = p_crow.shape[0] - 1
-    row = torch.repeat_interleave(torch.arange(n, device=p_col.device), (p_crow[1:] - p_crow[:-1]).long())
-    key = p_col.long() * n + row
-    return torch.argsort(key, stable=True).to(torch.int32)
+def _product(a, b, n_cols, out, missing):
+    """C = A B for CSR triples.  Without `out` (the set-up) the sort-based SpGEMM forms C's pattern and values.  With
+    `out`, the C that SpGEMM formed before (a refresh), the values are written into out's arrays in place and products
+    outside its pattern are counted into `missing`."""
+    if out is None:
+        return ops.csr_spgemm(a, b[0].shape[0] - 1, b, n_cols)
+    ops.csr_spgemm_numeric(a, b, out[0], out[1], out[2], missing)
+    return out
+
+
+def _transpose(p, n_coarse, out):
+    """(R, r_map) of R = P^T, whose entry k is P's entry r_map[k].  Without `out` (the set-up) both follow from P's
+    pattern: r_map is a stable sort of P's (column, row) keys, R's CSR order.  With `out` (a refresh) P is gathered into
+    out's R in place."""
+    if out is None:
+        n = p[0].shape[0] - 1
+        row = torch.repeat_interleave(torch.arange(n, device=p[1].device), (p[0][1:] - p[0][:-1]).long())
+        r_map = torch.argsort(p[1].long() * n + row, stable=True)
+        counts = torch.bincount(p[1].long(), minlength=n_coarse)
+        r_crow = torch.cat([counts.new_zeros(1), torch.cumsum(counts, 0)]).to(torch.int32)
+        out = ((r_crow, row[r_map].to(torch.int32), torch.empty_like(p[2])), r_map.to(torch.int32))
+    r, r_map = out
+    ops.gather_fill(r_map, p[2], 0.0, r[2])
+    return out
+
+
+def _level_values(a, diag, t, level, n_coarse, wdinv, out=None, missing=None):
+    """The values of one level from its operator `a`, its diagonal and its tentative prolongator `t` (CSR triples), in
+    this order: rho by power iteration, omega = 4 / (3 rho), omega D^-1 (into `wdinv`) and S = I - omega D^-1 A,
+    P = S T, R = P^T by gathering P through r_map, A P and A_c = R (A P).
+
+    The set-up passes no `out` and gets new patterns.  A refresh passes the level's (P, (R, r_map), A P, A_c); every
+    value is written into them in place.  Returns (rho, omega, P, R, r_map, A P, A_c)."""
+    rho = _spectral_radius(*a, 1.0 / diag, level)
+    omega = 4.0 / (3.0 * rho)
+    s_val = torch.empty_like(a[2])
+    ops.amg_smoother(*a, diag, omega, wdinv, s_val)
+    p_out, r_out, ap_out, c_out = out if out is not None else (None,) * 4
+    p = _product((a[0], a[1], s_val), t, n_coarse, p_out, missing)
+    r, r_map = _transpose(p, n_coarse, r_out)
+    ap = _product(a, p, n_coarse, ap_out, missing)
+    return rho, omega, p, r, r_map, ap, _product(r, ap, n_coarse, c_out, missing)
 
 
 def _dense_inverse(a_crow, a_col, a_val):
@@ -465,7 +479,8 @@ def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float 
     keep8 = None if keep is None else keep.reshape(-1).to(device=val.device, dtype=torch.uint8).contiguous()
     if keep8 is not None and keep8.shape[0] != n:
         raise ValueError("keep mask length does not match the matrix")
-    a = _masked_operator(crow, col, val, keep8)
+    m_crow, m_col, src = _masked_operator_map(crow, col, keep8)
+    a = (m_crow, m_col, ops.gather_fill(src, val, 1.0, val.new_empty(src.shape[0])))
     levels: List[AmgLevel] = []
     patterns: List[AmgLevelPattern] = []
     while a[0].shape[0] - 1 > max_coarse and len(levels) + 1 < max_levels:
@@ -481,22 +496,11 @@ def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float 
         t_crow = torch.cat([size.new_zeros(1), torch.cumsum(live.long(), 0)]).to(torch.int32)
         t_col = agg[live].contiguous()
         t_val = (1.0 / torch.sqrt(size[t_col.long()].to(a_val.dtype))).contiguous()
-        inv_diag = 1.0 / diag
-        rho = _spectral_radius(a_crow, a_col, a_val, inv_diag, level)
-        omega = 4.0 / (3.0 * rho)
-        wdinv = (omega / diag).contiguous()
-        row = torch.repeat_interleave(torch.arange(n_l, device=a_val.device), (a_crow[1:] - a_crow[:-1]).long())
-        s_val = ((row == a_col.long()).to(a_val.dtype) - wdinv[row] * a_val).contiguous()
-        p = ops.csr_spgemm((a_crow, a_col, s_val), n_l, (t_crow, t_col, t_val), n_agg)
-        r = ops.csr_spgemm(p, n_agg, transpose=True)
-        ap = ops.csr_spgemm(a, n_l, p, n_agg)
-        a_c = ops.csr_spgemm(r, n_l, ap, n_agg)
+        wdinv = torch.empty_like(diag)
+        rho, omega, p, r, r_map, ap, a_c = _level_values(a, diag, (t_crow, t_col, t_val), level, n_agg, wdinv)
         levels.append(AmgLevel(n_l, n_agg, a_crow, a_col, a_val, *p, *r, wdinv, agg, rho, omega))
         if refreshable:
-            r_map = _transpose_map(p[0], p[1])
-            if not torch.equal(p[2][r_map.long()].view(_bits(p[2].dtype)), r[2].view(_bits(r[2].dtype))):
-                raise RuntimeError("AMG set-up: R is not P^T gathered through the transpose map")
-            patterns.append(AmgLevelPattern(t_crow, t_col, t_val, ap[0], ap[1], ap[2], r_map))
+            patterns.append(AmgLevelPattern(t_crow, t_col, t_val, *ap, r_map))
         a = a_c
     a_crow, a_col, a_val = a
     n_c = a_crow.shape[0] - 1
@@ -507,12 +511,8 @@ def amg(matrix: torch.Tensor, keep: Optional[torch.Tensor] = None, theta: float 
     keep_all = torch.ones(n, dtype=torch.uint8, device=val.device) if keep8 is None else keep8.clone()
     pattern = None
     if refreshable:
-        pattern = AmgPattern(crow, col, _masked_operator_map(crow, col, keep8), patterns, a_crow, a_col, a_val)
+        pattern = AmgPattern(crow, col, src, patterns, a_crow, a_col, a_val)
     return AmgHierarchy(levels, coarse_inv, a_col.shape[0], keep_all, val.shape[0], theta, pattern=pattern)
-
-
-def _bits(dtype: torch.dtype) -> torch.dtype:
-    return torch.int64 if dtype == torch.float64 else torch.int32
 
 
 class _CgSolve(torch.autograd.Function):

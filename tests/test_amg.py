@@ -39,12 +39,23 @@ def _amg_aggregate(crow, col, strong, level):
     return torch.from_numpy(agg), n_agg
 
 
-def _csr_spgemm(a, n_cols_a, b=None, n_cols_b=0, transpose=False):
-    m = _csr(*a, n_cols_a)
-    m = m.T if transpose else m
-    if b is not None:
-        m = m @ _csr(*b, n_cols_b)
-    return _torch_csr(m, a[2].dtype)
+def _csr_spgemm(a, n_cols_a, b, n_cols_b):
+    return _torch_csr(_csr(*a, n_cols_a) @ _csr(*b, n_cols_b), a[2].dtype)
+
+
+def _amg_diag(crow, col, val):
+    return torch.from_numpy(_csr(crow, col, val, crow.shape[0] - 1).diagonal()).to(val.dtype)
+
+
+def _amg_smoother(crow, col, val, diag, omega, wdinv, s_val):
+    row = torch.repeat_interleave(torch.arange(crow.shape[0] - 1), (crow[1:] - crow[:-1]).long())
+    wdinv.copy_(omega / diag)
+    s_val.copy_((row == col.long()).to(val.dtype) - wdinv[row] * val)
+
+
+def _gather_fill(src, values, fill, out):
+    out.copy_(torch.where(src >= 0, values[src.long().clamp_min(0)], torch.full_like(out, fill)))
+    return out
 
 
 def _levels_of(h):
@@ -62,7 +73,7 @@ def _amg_vcycle(h, r):
 def install(monkeypatch):
     cpu_shim.install(monkeypatch)
     for name, fn in (("amg_strength", _amg_strength), ("amg_aggregate", _amg_aggregate), ("csr_spgemm", _csr_spgemm),
-                     ("amg_vcycle", _amg_vcycle)):
+                     ("amg_smoother", _amg_smoother), ("gather_fill", _gather_fill), ("amg_vcycle", _amg_vcycle)):
         monkeypatch.setattr(ops, name, fn)
 
 

@@ -12,7 +12,7 @@ import torch
 from oracle import amg_oracle as ao
 from pytorch_fem_solver_b200 import _lib, meshgen, ops, sparse
 from tests import amg_refresh_oracle as ro
-from tests.test_amg import _csr, as_matrix
+from tests.test_amg import _amg_diag, _csr, as_matrix
 from tests.test_amg import install as install_amg
 
 
@@ -33,25 +33,9 @@ def _csr_spgemm_numeric(a, b, c_crow, c_col, out=None, n_missing=None):
     return out, n_missing
 
 
-def _amg_diag(crow, col, val):
-    return torch.from_numpy(_csr(crow, col, val, crow.shape[0] - 1).diagonal()).to(val.dtype)
-
-
-def _amg_smoother(crow, col, val, diag, omega, wdinv, s_val):
-    row = torch.repeat_interleave(torch.arange(crow.shape[0] - 1), (crow[1:] - crow[:-1]).long())
-    wdinv.copy_(omega / diag)
-    s_val.copy_((row == col.long()).to(val.dtype) - wdinv[row] * val)
-
-
-def _gather_fill(src, values, fill, out):
-    out.copy_(torch.where(src >= 0, values[src.long().clamp_min(0)], torch.full_like(out, fill)))
-    return out
-
-
 def install(monkeypatch):
     install_amg(monkeypatch)
-    for name, fn in (("csr_spgemm_numeric", _csr_spgemm_numeric), ("amg_diag", _amg_diag), ("amg_smoother", _amg_smoother),
-                     ("gather_fill", _gather_fill)):
+    for name, fn in (("csr_spgemm_numeric", _csr_spgemm_numeric), ("amg_diag", _amg_diag)):
         monkeypatch.setattr(ops, name, fn)
 
 

@@ -131,6 +131,19 @@ def test_numeric_spgemm_counts_products_outside_the_pattern():
 
 # ---------------------------------------------------------------------------------------------- the refresh
 @pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
+def test_refreshable_setup_builds_the_same_hierarchy(dtype):
+    """amg(A) and amg(A, refreshable=True) give the same hierarchy bit for bit on the device (512 x 512)."""
+    k, keep, _, _ = problem(512, 512)
+    a, keep_t = _cuda_matrix(k, dtype), torch.from_numpy(keep).cuda()
+    plain, kept = sparse.amg(a, keep_t), sparse.amg(a, keep_t, refreshable=True)
+    assert plain.pattern is None and kept.pattern is not None
+    assert len(plain.levels) == len(kept.levels) >= 3
+    for t1, t2 in zip(hierarchy_tensors(plain), hierarchy_tensors(kept)):
+        assert _bitwise(t1, t2) if t1.is_floating_point() else (t1.dtype == t2.dtype and torch.equal(t1, t2))
+    assert plain.rho == kept.rho and plain.omega == kept.omega and plain.coarse_nnz == kept.coarse_nnz
+
+
+@pytest.mark.parametrize("dtype", [torch.float64, torch.float32])
 @pytest.mark.parametrize("masked", [True, False])
 def test_refresh_with_twice_the_matrix_is_a_fresh_build(dtype, masked):
     """amg(A).refresh(2 A) == amg(2 A) bit for bit: scaling by 2 is exact and the strength test, the power iteration and
