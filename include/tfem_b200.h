@@ -219,6 +219,21 @@ typedef struct tfem_amg_level {
                                     const T* frac_t, const tfem_bilinear* host_form,               \
                                     const tfem_source* host_source,                                \
                                     const T* f_q, T* local_mat, T* local_vec, void* stream);       \
+  /* The same local forms with coefficient fields sampled at the quadrature points:               \
+   * local_mat[e,i,j] = (grad phi_i . grad phi_j) det sum_q w_q alpha_q[e,q]                      \
+   *                  + det sum_q w_q beta_q[e,q] phi_i(q) phi_j(q)                  [n_el,3,3]   \
+   * (on a fracture: tangential 3-D gradients, det includes det J_f); local_vec exactly as        \
+   * tfem_tri_p1_local_forms writes it.  alpha_q, beta_q [n_el,n_q]; a NULL field takes the       \
+   * matching constant of host_form (which may then be NULL only if both fields are given). */    \
+  int tfem_tri_p1_weighted_local_forms_##SUF(int64_t n_el, int64_t n_el_per_mesh,                  \
+                                             int64_t n_vert_per_mesh, const T* coords,             \
+                                             const int32_t* conn, int quad_order,                  \
+                                             const T* frac_jac, const T* frac_inv,                 \
+                                             const T* frac_det, const T* frac_t,                   \
+                                             const tfem_bilinear* host_form,                       \
+                                             const tfem_source* host_source, const T* f_q,         \
+                                             const T* alpha_q, const T* beta_q, T* local_mat,      \
+                                             T* local_vec, void* stream);                          \
   /* Fused assembly to CSR + load vector in ONE pass over row tiles (BASELINE config 2):          \
    * csr_val[p] = sum over elements of alpha K_loc + beta M_loc, load[r] = sum of local loads,    \
    * each summed in increasing element order (deterministic, no atomics).  The tile plan is      \

@@ -83,6 +83,8 @@ _TYPED = {
     "tfem_scatter_bilinear": [I64, P, P, P, P, P],
     "tfem_scatter_linear": [I64, P, P, P, P, P],
     "tfem_tri_p1_local_forms": [I64, I64, I64, P, P, c_int, P, P, P, P, POINTER(Bilinear), POINTER(Source), P, P, P, P],
+    "tfem_tri_p1_weighted_local_forms": [I64, I64, I64, P, P, c_int, P, P, P, P, POINTER(Bilinear), POINTER(Source), P, P, P, P, P,
+                                         P],
     "tfem_tri_p1_assemble_csr": [POINTER(TilePlan), P, c_int, POINTER(Bilinear), POINTER(Source), P, P, P],
     "tfem_tri_p1_assemble_csr_ex": [POINTER(TilePlan), P, c_int, POINTER(Bilinear), POINTER(Source), P, I64, P, P, P, P],
     "tfem_weak_residual_local": [I64, I64, I64, P, P, c_int, P, P, P, P, POINTER(Source), P, P, P, P],

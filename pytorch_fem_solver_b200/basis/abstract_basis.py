@@ -204,7 +204,8 @@ class AbstractBasis(abc.ABC):
         """f at this basis' quadrature points, (N_total, n_q).  The points of a basis are fixed, so the samples of
         a `forms.SampledSource` are evaluated once per (source object, basis, geometry) and reused by every later
         call -- a training loop calls the residual thousands of times with the same right-hand side
-        (examples/example_weak.py:64-75).  `source.refresh()` drops them (a callable with changing state)."""
+        (examples/example_weak.py:64-75).  `source.refresh()` drops them (a callable with changing state).
+        Callable coefficients of a `forms.FusedBilinear` are `SampledSource`s too and share this cache."""
         lay = self._layout
         key = (id(self), self._geometry_version, self.dtype)
         cache = getattr(src, "_samples", None)
@@ -217,6 +218,34 @@ class AbstractBasis(abc.ABC):
             except AttributeError:  # a source type without attribute storage: evaluate every time
                 pass
         return cache[1]
+
+    def _coefficient_samples(self, coefficient) -> Optional[torch.Tensor]:
+        """(N_total, n_q) contiguous values of a field coefficient of a `forms.FusedBilinear`; None for a number."""
+        if isinstance(coefficient, float):
+            return None
+        if isinstance(coefficient, forms.SampledSource):
+            return self._sampled_source(coefficient)
+        lay = self._layout
+        return coefficient.detach().to(self.dtype).expand(*lay.lead, self.n_q, 1, 1).reshape(lay.n_total, self.n_q).contiguous()
+
+    def _check_coefficients(self, bilinear) -> None:
+        """Reject tensor coefficients the fused kernel cannot take, before anything is launched."""
+        target = (*self._layout.lead, self.n_q, 1, 1)
+        for name in ("alpha", "beta"):
+            c = getattr(bilinear, name)
+            if not isinstance(c, torch.Tensor):
+                continue
+            try:
+                shape = torch.broadcast_shapes(c.shape, target)
+            except RuntimeError:
+                shape = None
+            if shape != target:
+                raise ValueError(f"coefficient {name} of shape {tuple(c.shape)} does not broadcast to {target}")
+            if c.device != self.device:
+                raise ValueError(f"coefficient {name} is on {c.device}, the basis on {self.device}")
+            if c.requires_grad and torch.is_grad_enabled():
+                raise ValueError(f"coefficient {name} requires grad: the fused assembly does not differentiate with respect to "
+                                 "coefficients; use the generic route integrate_bilinear_form(lambda b: form(b)), which does")
 
     # ------------------------------------------------------------------ integrate_*
     def _reduce_integrand(self, integrand: torch.Tensor) -> torch.Tensor:
@@ -312,7 +341,8 @@ class AbstractBasis(abc.ABC):
         """Matrix and load vector of named forms in one pass (BASELINE config 2).
 
         `path`: "tiled" = single fused kernel over row tiles, "two_pass" = local_forms +
-        scatter kernels, "auto" = tiled for planar meshes with an analytic source."""
+        scatter kernels, "auto" = tiled for planar meshes with an analytic source.  A form with field
+        coefficients (see `forms.FusedBilinear`) always takes the two-pass path; "tiled" raises for it."""
         values, vec = self._assemble_fused(bilinear, load.source if load is not None else None, path)
         return (
             self._matrix_result(values, layout) if values is not None else None,
@@ -354,6 +384,8 @@ class AbstractBasis(abc.ABC):
         src = forms.as_source(source)
         want_mat = bilinear is not None
         want_vec = source is not None
+        if want_mat and bilinear.has_field:
+            return self._assemble_weighted(bilinear, src if want_vec else None, path)
         alpha, beta = (bilinear.alpha, bilinear.beta) if want_mat else (0.0, 0.0)
         sampled = want_vec and src.kind == ops.SRC_SAMPLED
         # one launch for everything but analytic (x, y) sources on fractures, which the kernels evaluate in 3-D
@@ -373,6 +405,25 @@ class AbstractBasis(abc.ABC):
             src.kind if want_vec else 0, list(src.params), f_q, *lay.frac_args(),
         )
         values = ops.scatter(local_mat.reshape(-1), pat.seg, pat.perm, self._inverse("bilinear")) if want_mat else None
+        vec = ops.scatter(local_vec.reshape(-1), pat.lin_seg, pat.lin_perm, self._inverse("linear")) if want_vec else None
+        return values, vec
+
+    def _assemble_weighted(self, bilinear, src, path: str):
+        """Field coefficients: `tfem_tri_p1_weighted_local_forms` (one launch) + the bilinear and linear scatters."""
+        if path == "tiled":
+            raise NotImplementedError("the tiled assembly takes constant coefficients; field coefficients run on path='two_pass'")
+        self._check_coefficients(bilinear)
+        lay, pat = self._layout, self.pattern
+        alpha_q, beta_q = self._coefficient_samples(bilinear.alpha), self._coefficient_samples(bilinear.beta)
+        alpha = bilinear.alpha if alpha_q is None else 0.0
+        beta = bilinear.beta if beta_q is None else 0.0
+        want_vec = src is not None
+        f_q = self._sampled_source(src) if want_vec and src.kind == ops.SRC_SAMPLED else None
+        local_mat, local_vec = ops.weighted_local_forms(
+            lay.coords, lay.conn, lay.n_el_per_mesh, lay.n_vert_per_mesh, self._element.integration_order, alpha, beta,
+            alpha_q, beta_q, src.kind if want_vec else 0, list(src.params) if want_vec else [0.0] * 4, f_q, *lay.frac_args(),
+        )
+        values = ops.scatter(local_mat.reshape(-1), pat.seg, pat.perm, self._inverse("bilinear"))
         vec = ops.scatter(local_vec.reshape(-1), pat.lin_seg, pat.lin_perm, self._inverse("linear")) if want_vec else None
         return values, vec
 
@@ -498,6 +549,8 @@ class HostPipeline:
         src = forms.as_source(load.source if load is not None else None)
         if lay.frac is not None or src.kind == ops.SRC_SAMPLED:
             raise NotImplementedError("the host pipeline drives the tiled kernel: planar mesh and analytic source")
+        if bilinear is not None and bilinear.has_field:
+            raise NotImplementedError("the host pipeline drives the tiled kernel, which takes constant coefficients only")
         self.basis, self.depth = basis, max(int(depth), 1)
         self.want_mat, self.want_vec = bilinear is not None, load is not None
         self.alpha, self.beta = (bilinear.alpha, bilinear.beta) if self.want_mat else (0.0, 0.0)

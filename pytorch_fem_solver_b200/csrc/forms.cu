@@ -35,6 +35,59 @@ struct FracLite {
   const T* t;    // [n_mesh,3]
 };
 
+// Gradients of the three P1 shape functions of an element: the planar ones, or on a fracture the tangential
+// 3-D ones g_i J_f^+ (fracture_basis.py:20-22).  Planar rows have gr[i][2] = 0.
+template <typename T, bool FRAC>
+__device__ __forceinline__ void p1_gradients(const TriGeom<T>& g, const FracLite<T>& frac, int mesh, T gr[3][3]) {
+  gr[0][0] = -g.i00 - g.i10; gr[0][1] = -g.i01 - g.i11; gr[0][2] = T(0);
+  gr[1][0] = g.i00;          gr[1][1] = g.i01;          gr[1][2] = T(0);
+  gr[2][0] = g.i10;          gr[2][1] = g.i11;          gr[2][2] = T(0);
+  if constexpr (FRAC) {
+    T jinv[2][3];
+#pragma unroll
+    for (int a = 0; a < 2; ++a)
+#pragma unroll
+      for (int c = 0; c < 3; ++c) jinv[a][c] = __ldg(frac.inv + 6 * mesh + 3 * a + c);
+#pragma unroll
+    for (int i = 0; i < 3; ++i) {
+      const T a0 = gr[i][0], a1 = gr[i][1];
+#pragma unroll
+      for (int c = 0; c < 3; ++c) gr[i][c] = a0 * jinv[0][c] + a1 * jinv[1][c];
+    }
+  }
+}
+
+// Local load vector b_i = sum_q w_q det f(x_q) phi_i(q) over the first n_q points of `quad`, term for term the loop of
+// local_forms_kernel.  `sampled(q)` gives f at point q of a TFEM_SRC_SAMPLED source; analytic sources are evaluated
+// at the mapped point (on a fracture at its first two 3-D coordinates).  local_forms_kernel keeps its own copy of the
+// loop: calling this helper there reorders the instructions of its fracture instantiations.
+template <typename T, bool FRAC, typename Sampled>
+__device__ __forceinline__ void p1_load(const QuadT<T>& quad, int n_q, T x0, T y0, T x1, T y1, T x2, T y2, T det, const SourceT<T>& src,
+                                        const FracLite<T>& frac, int mesh, Sampled sampled, T& b0, T& b1, T& b2) {
+  b0 = T(0), b1 = T(0), b2 = T(0);
+  if (src.kind == TFEM_SRC_NONE) return;
+  for (int q = 0; q < n_q; ++q) {
+    T f;
+    if (src.kind == TFEM_SRC_SAMPLED) {
+      f = sampled(q);
+    } else {
+      T px = quad.l0[q] * x0 + quad.l1[q] * x1 + quad.l2[q] * x2;
+      T py = quad.l0[q] * y0 + quad.l1[q] * y1 + quad.l2[q] * y2;
+      if constexpr (FRAC) {  // analytic sources see the first two 3-D coordinates
+        const T X = __ldg(frac.jac + 6 * mesh + 0) * px + __ldg(frac.jac + 6 * mesh + 1) * py + __ldg(frac.t + 3 * mesh);
+        const T Y = __ldg(frac.jac + 6 * mesh + 2) * px + __ldg(frac.jac + 6 * mesh + 3) * py + __ldg(frac.t + 3 * mesh + 1);
+        px = X;
+        py = Y;
+      }
+      f = source_eval(src, px, py);
+    }
+    const T wf = quad.w[q] * det * f;
+    b0 += wf * quad.l0[q];
+    b1 += wf * quad.l1[q];
+    b2 += wf * quad.l2[q];
+  }
+}
+
 // ---------------------------------------------------------------------------------------------
 // Fused local forms, one thread per element.
 //   local_mat[e,i,j] = alpha * (grad phi_i . grad phi_j) * sum_q dx_q + beta * det * mref[i][j]
@@ -66,22 +119,7 @@ __global__ void __launch_bounds__(256) local_forms_kernel(
 
   if (local_mat) {
     T gr[3][3];
-    gr[0][0] = -g.i00 - g.i10; gr[0][1] = -g.i01 - g.i11; gr[0][2] = T(0);
-    gr[1][0] = g.i00;          gr[1][1] = g.i01;          gr[1][2] = T(0);
-    gr[2][0] = g.i10;          gr[2][1] = g.i11;          gr[2][2] = T(0);
-    if constexpr (FRAC) {
-      T jinv[2][3];
-#pragma unroll
-      for (int a = 0; a < 2; ++a)
-#pragma unroll
-        for (int c = 0; c < 3; ++c) jinv[a][c] = __ldg(frac.inv + 6 * mesh + 3 * a + c);
-#pragma unroll
-      for (int i = 0; i < 3; ++i) {
-        const T a0 = gr[i][0], a1 = gr[i][1];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) gr[i][c] = a0 * jinv[0][c] + a1 * jinv[1][c];
-      }
-    }
+    p1_gradients<T, FRAC>(g, frac, mesh, gr);
     const T area = quad.wsum * det;  // sum_q dx_q
     T* out = local_mat + 9 * (int64_t)e;
 #pragma unroll
@@ -118,6 +156,92 @@ __global__ void __launch_bounds__(256) local_forms_kernel(
         b2 += wf * quad.l2[q];
       }
     }
+    T* out = local_vec + 3 * (int64_t)e;
+    out[0] = b0;
+    out[1] = b1;
+    out[2] = b2;
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Fused local forms with coefficient fields sampled at the quadrature points:
+//   local_mat[e,i,j] = (grad phi_i . grad phi_j) det sum_q w_q alpha_q + det sum_q w_q beta_q phi_i(q) phi_j(q)
+//   local_vec[e,i]   = as local_forms_kernel
+// alpha_q / beta_q [n_el, NQ] (NULL: the constant alpha / beta) and f_q are NQ-strided per element; the rows of a
+// block of kStagedBlock elements are staged through shared memory with coalesced loads, as in the residual kernel.
+// ---------------------------------------------------------------------------------------------
+template <typename T, bool FRAC, int NQ>
+__global__ void __launch_bounds__(kStagedBlock) weighted_local_forms_kernel(
+    int n_el, int n_el_per_mesh, int n_vert_per_mesh, const T* __restrict__ coords,
+    const int32_t* __restrict__ conn, const QuadT<T> quad, const FracLite<T> frac, T alpha, T beta,
+    const SourceT<T> src, const T* __restrict__ f_q, const T* __restrict__ alpha_q, const T* __restrict__ beta_q,
+    T* __restrict__ local_mat, T* __restrict__ local_vec) {
+  constexpr int ROWP = NQ | 1;  // odd stride: conflict-free rows
+  __shared__ T s_a[kStagedBlock * ROWP];
+  __shared__ T s_b[kStagedBlock * ROWP];
+  __shared__ T s_f[kStagedBlock * ROWP];
+  const int e0 = blockIdx.x * kStagedBlock;
+  const int count = min(kStagedBlock, n_el - e0);
+  const bool field_a = local_mat && alpha_q, field_b = local_mat && beta_q;
+  const bool sampled = local_vec && src.kind == TFEM_SRC_SAMPLED;
+  for (int i = threadIdx.x; i < count * NQ; i += kStagedBlock) {
+    const int at = (i / NQ) * ROWP + i % NQ;
+    const int64_t from = (int64_t)e0 * NQ + i;
+    if (field_a) s_a[at] = __ldg(alpha_q + from);
+    if (field_b) s_b[at] = __ldg(beta_q + from);
+    if (sampled) s_f[at] = __ldg(f_q + from);
+  }
+  __syncthreads();
+  const int e = e0 + threadIdx.x;
+  if (e >= n_el) return;
+  const int mesh = e / n_el_per_mesh;
+  const int64_t voff = (int64_t)mesh * n_vert_per_mesh;
+  const int v0 = __ldg(conn + 3 * (int64_t)e + 0);
+  const int v1 = __ldg(conn + 3 * (int64_t)e + 1);
+  const int v2 = __ldg(conn + 3 * (int64_t)e + 2);
+  T x0, y0, x1, y1, x2, y2;
+  load_xy(coords, voff + v0, x0, y0);
+  load_xy(coords, voff + v1, x1, y1);
+  load_xy(coords, voff + v2, x2, y2);
+  const TriGeom<T> g = tri_geom(x0, y0, x1, y1, x2, y2);
+  T detf = T(1);
+  if constexpr (FRAC) detf = __ldg(frac.det + mesh);
+  const T det = g.det * detf;
+  const int row = threadIdx.x * ROWP;
+
+  if (local_mat) {
+    T gr[3][3];
+    p1_gradients<T, FRAC>(g, frac, mesh, gr);
+    T wa = T(0);
+    T m[6] = {};  // sum_q w_q beta_q phi_i phi_j: 00 11 22 01 12 02
+#pragma unroll
+    for (int q = 0; q < NQ; ++q) {
+      wa += quad.w[q] * (field_a ? s_a[row + q] : alpha);
+      const T wb = quad.w[q] * (field_b ? s_b[row + q] : beta);
+      const T l0 = quad.l0[q], l1 = quad.l1[q], l2 = quad.l2[q];
+      m[0] += wb * (l0 * l0);
+      m[1] += wb * (l1 * l1);
+      m[2] += wb * (l2 * l2);
+      m[3] += wb * (l0 * l1);
+      m[4] += wb * (l1 * l2);
+      m[5] += wb * (l0 * l2);
+    }
+    const T stiff = wa * det;
+    const T mass[9] = {m[0], m[3], m[5], m[3], m[1], m[4], m[5], m[4], m[2]};
+    T* out = local_mat + 9 * (int64_t)e;
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+      for (int j = 0; j < 3; ++j) {
+        T dot = gr[i][0] * gr[j][0] + gr[i][1] * gr[j][1];
+        if constexpr (FRAC) dot += gr[i][2] * gr[j][2];
+        out[3 * i + j] = dot * stiff + mass[3 * i + j] * det;
+      }
+  }
+
+  if (local_vec) {
+    T b0, b1, b2;
+    p1_load<T, FRAC>(quad, NQ, x0, y0, x1, y1, x2, y2, det, src, frac, mesh, [&](int q) { return s_f[row + q]; }, b0, b1, b2);
     T* out = local_vec + 3 * (int64_t)e;
     out[0] = b0;
     out[1] = b1;
@@ -483,6 +607,41 @@ int local_forms(int64_t n_el, int64_t n_el_per_mesh, int64_t n_vert_per_mesh, co
 }
 
 template <typename T>
+int weighted_local_forms(int64_t n_el, int64_t n_el_per_mesh, int64_t n_vert_per_mesh, const T* coords,
+                         const int32_t* conn, int quad_order, const T* frac_jac, const T* frac_det, const T* frac_t,
+                         const T* frac_inv, const tfem_bilinear* form, const tfem_source* source, const T* f_q,
+                         const T* alpha_q, const T* beta_q, T* local_mat, T* local_vec, void* stream) {
+  if (n_el < 0 || n_el_per_mesh <= 0 || n_vert_per_mesh <= 0) return TFEM_ERR_BAD_ARG;
+  if (n_el == 0) return TFEM_OK;
+  if (!coords || !conn) return TFEM_ERR_BAD_ARG;
+  if (local_mat && !form && (!alpha_q || !beta_q)) return TFEM_ERR_BAD_ARG;
+  if (n_el > kMaxIndex / 9) return TFEM_ERR_TOO_LARGE;
+  if (tri_n_q(quad_order) == 0) return TFEM_ERR_UNSUPPORTED;
+  const SourceT<T> src = make_source<T>(source);
+  if (src.kind < TFEM_SRC_NONE || src.kind > TFEM_SRC_SINSIN) return TFEM_ERR_BAD_ARG;
+  if (local_vec && src.kind == TFEM_SRC_SAMPLED && !f_q) return TFEM_ERR_BAD_ARG;
+  const bool frac = frac_det != nullptr;
+  if (frac && (!frac_inv || !frac_jac || !frac_t)) return TFEM_ERR_BAD_ARG;
+  const QuadT<T> quad = make_quad<T>(quad_order);
+  const FracLite<T> fl{frac_jac, frac_inv, frac_det, frac_t};
+  const T alpha = form ? T(form->alpha) : T(0), beta = form ? T(form->beta) : T(0);
+  auto s = static_cast<cudaStream_t>(stream);
+  const unsigned blocks = blocks_for(n_el, kStagedBlock);
+#define TFEM_LAUNCH_WEIGHTED(F, Q)                                                                                  \
+  weighted_local_forms_kernel<T, F, Q><<<blocks, kStagedBlock, 0, s>>>((int)n_el, (int)n_el_per_mesh, (int)n_vert_per_mesh, \
+                                                                      coords, conn, quad, fl, alpha, beta, src, f_q, alpha_q, \
+                                                                      beta_q, local_mat, local_vec)
+  switch (quad.n_q) {
+    case 1: if (frac) TFEM_LAUNCH_WEIGHTED(true, 1); else TFEM_LAUNCH_WEIGHTED(false, 1); break;
+    case 3: if (frac) TFEM_LAUNCH_WEIGHTED(true, 3); else TFEM_LAUNCH_WEIGHTED(false, 3); break;
+    case 4: if (frac) TFEM_LAUNCH_WEIGHTED(true, 4); else TFEM_LAUNCH_WEIGHTED(false, 4); break;
+    default: if (frac) TFEM_LAUNCH_WEIGHTED(true, 6); else TFEM_LAUNCH_WEIGHTED(false, 6); break;
+  }
+#undef TFEM_LAUNCH_WEIGHTED
+  return check_launch();
+}
+
+template <typename T>
 int weak_residual_local(int64_t n_el, int64_t n_el_per_mesh, int64_t n_vert_per_mesh, const T* coords,
                         const int32_t* conn, int quad_order, const T* frac_jac, const T* frac_inv,
                         const T* frac_det, const T* frac_t, const tfem_source* source, const T* f_q,
@@ -559,6 +718,16 @@ int weak_residual_bwd(int64_t n_el, int64_t n_el_per_mesh, int64_t n_vert_per_me
     return tfem::local_forms<T>(n_el, n_el_per_mesh, n_vert_per_mesh, coords, conn, quad_order,     \
                                 frac_jac, frac_det, frac_t, frac_inv, host_form, host_source, f_q,  \
                                 local_mat, local_vec, stream);                                      \
+  }                                                                                                 \
+  extern "C" int tfem_tri_p1_weighted_local_forms_##SUF(                                            \
+      int64_t n_el, int64_t n_el_per_mesh, int64_t n_vert_per_mesh, const T* coords,                \
+      const int32_t* conn, int quad_order, const T* frac_jac, const T* frac_inv, const T* frac_det, \
+      const T* frac_t, const tfem_bilinear* host_form, const tfem_source* host_source,              \
+      const T* f_q, const T* alpha_q, const T* beta_q, T* local_mat, T* local_vec, void* stream) {  \
+    return tfem::weighted_local_forms<T>(n_el, n_el_per_mesh, n_vert_per_mesh, coords, conn,        \
+                                         quad_order, frac_jac, frac_det, frac_t, frac_inv,          \
+                                         host_form, host_source, f_q, alpha_q, beta_q, local_mat,   \
+                                         local_vec, stream);                                        \
   }                                                                                                 \
   extern "C" int tfem_weak_residual_local_##SUF(                                                    \
       int64_t n_el, int64_t n_el_per_mesh, int64_t n_vert_per_mesh, const T* coords,                \

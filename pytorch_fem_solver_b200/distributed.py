@@ -672,6 +672,8 @@ class PartitionedFractureAssembly:
 
         src = forms.as_source(source)
         want_mat, want_vec = bilinear is not None, source is not None
+        if want_mat and bilinear.has_field:
+            raise NotImplementedError("the distributed assembly runs the tiled kernel, which takes constant coefficients only")
         f_q = None
         if want_vec and src.kind == ops.SRC_SAMPLED:
             f_q = self.basis._sampled_source(src)[self.lo : self.hi].contiguous()

@@ -12,6 +12,11 @@ Forms covered (SURVEY.md section 8(a) row a15):
   WeakResidual(source)               examples/example_weak.py:64-75, example_patches.py:102-113,
                                      example_fracture_vpinns.py:104-113
   H1Error(exact, exact_grad)         examples/example_weak.py:113-124
+
+Coefficients: `Stiffness(kappa)`, `Mass(c)` and `StiffnessMass(kappa, c)` take numbers, callables of the quadrature
+points or tensors broadcastable to `(*lead, n_q, 1, 1)` (DESIGN.md section 8(g)), so `-div(kappa grad u) + c u = f`
+assembles without an integrand.  The VPINN residual of `-div(kappa grad u) = f` needs no new kernel: pass
+`kappa_q * grad u_NN` as the gradient to `WeakResidual`.
 """
 
 from __future__ import annotations
@@ -84,18 +89,49 @@ def as_source(source) -> Source:
     return ConstSource(float(source))
 
 
-class FusedBilinear:
-    """alpha * grad(u).grad(v) + beta * u v."""
+def _coefficient(value):
+    """A number stays a float (the constant-coefficient kernels); a tensor is kept as given; a callable of the
+    quadrature points is wrapped in a `SampledSource`, whose samples the basis caches like a sampled right-hand side."""
+    if isinstance(value, torch.Tensor) and value.dim() > 0:
+        return value
+    if callable(value):
+        return SampledSource(value)
+    return float(value)
 
-    def __init__(self, alpha: float = 0.0, beta: float = 0.0):
-        self.alpha, self.beta = float(alpha), float(beta)
+
+def _is_zero(coefficient) -> bool:
+    return isinstance(coefficient, float) and coefficient == 0.0
+
+
+class FusedBilinear:
+    """alpha * grad(u).grad(v) + beta * u v.
+
+    `alpha` and `beta` each take a number, a callable of the quadrature points returning `(..., 1)` values, or a
+    tensor broadcastable to `(*lead, n_q, 1, 1)` (`lead` = the basis' element batch shape: `(N, 1, 1, 1)` per element,
+    `(N, n_q, 1, 1)` per quadrature point, `(F, 1, 1, 1, 1)` per fracture).  Field coefficients run on the two-pass
+    path (`tfem_tri_p1_weighted_local_forms`); number coefficients keep the constant-coefficient kernels."""
+
+    def __init__(self, alpha=0.0, beta=0.0):
+        self.alpha, self.beta = _coefficient(alpha), _coefficient(beta)
+
+    @property
+    def has_field(self) -> bool:
+        """True when alpha or beta is a callable or tensor field rather than a number."""
+        return not (isinstance(self.alpha, float) and isinstance(self.beta, float))
+
+    def refresh(self):
+        """Forget the cached samples of callable coefficients (for callables whose values change between calls)."""
+        for c in (self.alpha, self.beta):
+            if isinstance(c, SampledSource):
+                c.refresh()
 
     def __call__(self, basis):
+        alpha, beta = (c(basis.integration_points) if isinstance(c, SampledSource) else c for c in (self.alpha, self.beta))
         out = None
-        if self.alpha != 0.0:
-            out = self.alpha * (basis.v_grad @ basis.v_grad.mT)
-        if self.beta != 0.0:
-            mass = self.beta * (basis.v @ basis.v.mT)
+        if not _is_zero(alpha):
+            out = alpha * (basis.v_grad @ basis.v_grad.mT)
+        if not _is_zero(beta):
+            mass = beta * (basis.v @ basis.v.mT)
             out = mass if out is None else out + mass
         if out is None:
             out = 0.0 * (basis.v @ basis.v.mT)
@@ -103,17 +139,17 @@ class FusedBilinear:
 
 
 class Stiffness(FusedBilinear):
-    def __init__(self, alpha: float = 1.0):
+    def __init__(self, alpha=1.0):
         super().__init__(alpha, 0.0)
 
 
 class Mass(FusedBilinear):
-    def __init__(self, beta: float = 1.0):
+    def __init__(self, beta=1.0):
         super().__init__(0.0, beta)
 
 
 class StiffnessMass(FusedBilinear):
-    def __init__(self, alpha: float = 1.0, beta: float = 1.0):
+    def __init__(self, alpha=1.0, beta=1.0):
         super().__init__(alpha, beta)
 
 

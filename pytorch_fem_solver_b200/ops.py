@@ -453,6 +453,52 @@ def _(coords, conn, n_el_per_mesh, n_vert_per_mesh, quad_order, alpha, beta, wan
     return coords.new_empty((n_el if want_matrix else 0, 3, 3)), coords.new_empty((n_el if source_kind else 0, 3))
 
 
+@torch.library.custom_op(f"{NS}::weighted_local_forms", mutates_args=())
+def weighted_local_forms(
+    coords: Tensor,
+    conn: Tensor,
+    n_el_per_mesh: int,
+    n_vert_per_mesh: int,
+    quad_order: int,
+    alpha: float,
+    beta: float,
+    alpha_q: Optional[Tensor],
+    beta_q: Optional[Tensor],
+    source_kind: int,
+    source_p: List[float],
+    f_q: Optional[Tensor] = None,
+    frac_jac: Optional[Tensor] = None,
+    frac_inv: Optional[Tensor] = None,
+    frac_det: Optional[Tensor] = None,
+    frac_t: Optional[Tensor] = None,
+) -> Tuple[Tensor, Tensor]:
+    """Per-element K(alpha_q) + M(beta_q) (N,3,3) and load (N,3); alpha_q / beta_q (N, n_q) or None for the constants."""
+    device = check_cuda(coords, conn, alpha_q, beta_q, f_q, frac_jac, frac_inv, frac_det, frac_t)
+    n_q = _nq_tri(quad_order)
+    n_el = conn.shape[0]
+    for name, field in (("alpha_q", alpha_q), ("beta_q", beta_q)):
+        if field is not None and (tuple(field.shape) != (n_el, n_q) or field.dtype != coords.dtype):
+            raise TfemError(f"{name} must be ({n_el}, {n_q}) {coords.dtype}, got {tuple(field.shape)} {field.dtype}")
+    opts = dict(dtype=coords.dtype, device=device)
+    want_vec = source_kind != _lib.TFEM_SRC_NONE
+    local_mat = torch.empty((n_el, 3, 3), **opts)
+    local_vec = torch.empty((n_el, 3) if want_vec else (0, 3), **opts)
+    call(
+        "tfem_tri_p1_weighted_local_forms", coords.dtype, device, n_el, n_el_per_mesh, n_vert_per_mesh, ptr(coords), ptr(conn),
+        quad_order, ptr(frac_jac), ptr(frac_inv), ptr(frac_det), ptr(frac_t), Bilinear(alpha, beta),
+        make_source(source_kind, source_p), ptr(f_q), ptr(alpha_q), ptr(beta_q), ptr(local_mat),
+        ptr(local_vec) if want_vec else None,
+    )
+    return local_mat, local_vec
+
+
+@weighted_local_forms.register_fake
+def _(coords, conn, n_el_per_mesh, n_vert_per_mesh, quad_order, alpha, beta, alpha_q, beta_q, source_kind, source_p,
+      f_q=None, frac_jac=None, frac_inv=None, frac_det=None, frac_t=None):
+    n_el = conn.shape[0]
+    return coords.new_empty((n_el, 3, 3)), coords.new_empty((n_el if source_kind else 0, 3))
+
+
 def _tiled_struct(tile_list: Tensor, tile_desc: Tensor, inst_blob: Tensor, tpl_desc: Tensor, tpl_blob: Tensor, meta: List[int],
                   progress: Optional[Tensor]):
     """struct tfem_tile_plan from the plan's device arrays and its integer fields (TilePlan.op_args)."""
